@@ -19,6 +19,11 @@ Workloads (BASELINE.json configs):
 `--impl reference` times the reference's OWN CPU implementation (the unmodified sources staged under
 baseline/_ref by tools/fetch_ref.py; the CPU oracle port when they are absent) on all host cores: sampling
 through model.generate and the G+D step through train_fns.GAN_training_function, one event per step.
+
+`--dump-outputs DIR` (sample / train workloads) writes what the timed paths returned in their last step as
+DIR/<name>.npy: the images of the sampling step, as many as DUMP_BYTES holds, picked with a fixed seed (device
+output and the post-processed host copy of the end-to-end path), and the five floats of the train step.  Inputs and weights
+come from fixed seeds, so two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -39,6 +44,21 @@ G_FWD_BYTES_PER_EVENT = 2.03e9
 G_FWD_FLOP_PER_EVENT = 0.134e12
 TRAIN_BYTES_PER_EVENT = 31.2e9
 TRAIN_FLOP_PER_EVENT = 1.73e12
+DUMP_BYTES = 32 << 20  # float32 bytes of the dumped images (both sampling arrays): 64 images at 256x256
+
+
+def dump_pick(n, image_bytes):
+    """The fixed, seeded choice of images of a batch of n that --dump-outputs writes."""
+    g = torch.Generator().manual_seed(0)
+    return torch.randperm(n, generator=g)[:max(1, DUMP_BYTES // image_bytes)].sort().values
+
+
+def write_dump(path, arrays):
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    for name, v in arrays.items():
+        a = v.detach().cpu().double().numpy() if v.dtype == torch.float64 else v.detach().cpu().float().numpy()
+        np.save(os.path.join(path, name + ".npy"), a)
 
 
 def peaks():
@@ -354,9 +374,8 @@ def run_reference(args, cfg):
         return
     t0 = time.perf_counter()
     train = args.workload == "train"
-    # bounded samples: ~3 s per sampling call, ~25-30 s per train step on a 16-thread host
-    k_s = max(1, min(args.steps, 10))
-    k_t = max(1, min(args.steps, 3 if train else 2))
+    # --steps sets both samples: ~3 s per sampling call, ~25-30 s per train step on a 16-thread host
+    k_s = k_t = max(1, args.steps)
     r = cpu_reference(cfg, k_s, k_t, train_warm=1)
     vs, vt = 1.0 / r["sample_s"], 1.0 / r["train_s"]
     cb_s = {"value": round(vs, 4), "unit": "events/s", "cores": r["cores"], "kind": r["kind"], "sample": r["sample_desc"]}
@@ -427,7 +446,8 @@ def stock_torch_gpu(cfg, dev):
 
 
 # ---------------------------------------------------------------------------------------- GPU workloads
-def bench_sample(args, cfg, dev, world, dist_on, ev, K_, W, hbm_peak):
+def bench_sample(args, cfg, dev, world, dist_on, ev, K_, W, hbm_peak, dump=None):
+    """dump: dict that receives the images of the last timed step (device path and end-to-end path)."""
     from iea_gan_b200 import engine as E_
     res_w = 256 * cfg["H_base"]
     G, _ = build_nets(cfg, dev, False)
@@ -436,9 +456,14 @@ def bench_sample(args, cfg, dev, world, dist_on, ev, K_, W, hbm_peak):
     z = torch.randn(n, cfg["dim_z"], device=dev)
     y = torch.arange(40, device=dev).repeat(ev)
 
+    last = {}
+
     def step():
         with torch.no_grad():
-            return G(z, y)
+            img = G(z, y)
+        if dump is not None:
+            last["img"] = img
+        return img
     step()
     torch.cuda.synchronize()
     l0 = E_.LAUNCHES[0]
@@ -465,6 +490,10 @@ def bench_sample(args, cfg, dev, world, dist_on, ev, K_, W, hbm_peak):
         post.record_stream(copy_stream)
         turn[0] += 1
     ms_e = timed(step_e2e, K_, W, dist_on, finish=lambda: torch.cuda.current_stream().wait_stream(copy_stream))
+    if dump is not None:
+        pick = dump_pick(n, (256 + 250) * res_w * 4)
+        dump["sample_images"] = last.pop("img")[pick.to(dev)]
+        dump["sample_e2e_images"] = outh[(turn[0] - 1) & 1][pick]
     hb = cfg["H_base"]
     gb = G_FWD_BYTES_PER_EVENT * ev * hb
     out = {"metric": "G-sample events/s (40 PXD imgs/event)", "value": round(value, 2), "unit": "events/s",
@@ -482,7 +511,8 @@ def bench_sample(args, cfg, dev, world, dist_on, ev, K_, W, hbm_peak):
     return out
 
 
-def bench_train(args, cfg, dev, world, dist_on, ev, K_, W, hbm_peak, graph):
+def bench_train(args, cfg, dev, world, dist_on, ev, K_, W, hbm_peak, graph, dump=None, prefix="train"):
+    """dump: dict that receives the five floats of the last timed step of the device-resident path."""
     import iea_gan_b200 as P
     from iea_gan_b200 import engine as E_
     from iea_gan_b200 import dp
@@ -509,7 +539,14 @@ def bench_train(args, cfg, dev, world, dist_on, ev, K_, W, hbm_peak, graph):
     # (the caching allocator needs ~10 full G+D steps to stop growing: warm up that long before timing)
     wt = max(W, 10)
     l0 = E_.LAUNCHES[0]
-    ms_t, spread = timed(lambda: train(x, y), K_, wt, dist_on, per_step=True)
+    last = {}
+
+    def step():
+        last["losses"] = train(x, y)
+    ms_t, spread = timed(step, K_, wt, dist_on, per_step=True)
+    if dump is not None:
+        for k, v in last["losses"].items():
+            dump["%s_%s" % (prefix, k)] = torch.tensor(v, dtype=torch.float64)
     launches_t = getattr(train, "launches_per_step", None) or (E_.LAUNCHES[0] - l0) // (K_ + wt)
     ms_te = timed(lambda: train(xh.to(dev, non_blocking=True), yh.to(dev, non_blocking=True)), K_, 3, dist_on)
     hb = cfg["H_base"]
@@ -652,7 +689,11 @@ def main():
     ap.add_argument("--sweep", default="1,4,16,64,256", help="event counts of --workload attn-sweep")
     ap.add_argument("--no-graph", action="store_true", help="train step launched kernel by kernel instead of as a CUDA graph")
     ap.add_argument("--no-extras", action="store_true", help="skip the cpu baselines / rooflines / extra workloads")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed step of the sample / train paths to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl != "b200" or args.workload == "attn-sweep"):
+        raise SystemExit("--dump-outputs covers the b200 sample and train workloads")
     from iea_gan_b200.default_config import shipped_config
     cfg = shipped_config(H_base=args.hbase, clip_norm=1e9)  # clip_norm: otherwise G never steps (train_fns.py:190)
     if args.impl == "reference":
@@ -681,6 +722,7 @@ def main():
     sampler = ClockSampler(local)
     sampler.start()
     extras = rank == 0 and world == 1 and not args.no_extras
+    dump = {} if args.dump_outputs and rank == 0 else None
 
     if args.workload == "attn-sweep":
         rows = bench_attn_sweep(args, cfg, dev, hbm_peak, tf_burst)
@@ -697,7 +739,7 @@ def main():
         return
 
     if args.workload == "sample":
-        s = bench_sample(args, cfg, dev, world, dist_on, args.events or 16, K_, W, hbm_peak)
+        s = bench_sample(args, cfg, dev, world, dist_on, args.events or 16, K_, W, hbm_peak, dump=dump)
         line = dict(common, **s)
         line["config"] = {"workload": "Generator sampling (RRM + ccbn + SNConv2d), %d events/GPU, 256x%d, train-mode BN, "
                                       "random-init weights" % (s["events_per_gpu"], res_w),
@@ -705,7 +747,8 @@ def main():
                           "l2": "per-step working set (>1 GB of activations) far exceeds the 126 MB L2"}
         line["clocks"] = sampler.summary()
         if not args.no_extras:
-            line["train_step"] = bench_train(args, cfg, dev, world, dist_on, 8, max(K_, 20), W, hbm_peak, graph)
+            line["train_step"] = bench_train(args, cfg, dev, world, dist_on, 8, K_, W, hbm_peak, graph, dump=dump,
+                                             prefix="train_step")
     else:
         ev_t = args.events or 8
         if args.global_events:
@@ -713,7 +756,7 @@ def main():
                 raise SystemExit("--global-events %d does not split over %d ranks" % (args.global_events, world))
             ev_t = args.global_events // world
             common["scaling"] = "strong"
-        t = bench_train(args, cfg, dev, world, dist_on, ev_t, K_, W, hbm_peak, graph)
+        t = bench_train(args, cfg, dev, world, dist_on, ev_t, K_, W, hbm_peak, graph, dump=dump)
         line = dict(common, **t)
         if args.global_events:
             line["global_events"] = args.global_events
@@ -727,7 +770,7 @@ def main():
         try:
             if args.hbase == 1 and args.workload == "sample":
                 c3 = dict(cfg, H_base=3)
-                h3 = bench_sample(args, c3, dev, world, False, 8, min(K_, 10), W, hbm_peak)
+                h3 = bench_sample(args, c3, dev, world, False, 8, K_, W, hbm_peak)
                 line["hbase3"] = {k: h3[k] for k in ("value", "unit", "ms_per_step", "events_per_gpu", "e2e", "step_roofline")}
                 line["hbase3"]["workload"] = "Generator sampling at the shipped geometry 256x768 (H_base=3), 8 events"
         except Exception as e:
@@ -764,6 +807,8 @@ def main():
                     line["train_step"]["cpu_baseline"] = cb_t
         except Exception as e:
             line["cpu_baseline"] = {"error": repr(e)}
+    if dump is not None:
+        write_dump(args.dump_outputs, dump)
     if rank == 0:
         print(json.dumps(line), flush=True)
     if dist_on:

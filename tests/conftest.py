@@ -7,6 +7,8 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
 GOLDEN = os.path.join(ROOT, "tests", "golden")
+sys.path.insert(0, GOLDEN)
+from golden_io import load_golden  # noqa: E402
 
 
 def pytest_configure(config):
@@ -22,11 +24,14 @@ def small_cfg():
 
 @pytest.fixture(scope="session")
 def golden_fwd():
-    import torch
-    return torch.load(os.path.join(GOLDEN, "small_fwd.pt"))
+    return load_golden(os.path.join(GOLDEN, "small_fwd"))
 
 
 @pytest.fixture(scope="session")
 def golden_step():
-    import torch
-    return torch.load(os.path.join(GOLDEN, "small_step.pt"))
+    return load_golden(os.path.join(GOLDEN, "small_step"))
+
+
+@pytest.fixture(scope="session")
+def golden_modules():
+    return load_golden(os.path.join(GOLDEN, "modules"))

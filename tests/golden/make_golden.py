@@ -9,11 +9,12 @@ It writes small fixtures next to this file:
   small_cfg.json        the reduced configuration (resolution 64, G_ch 16, D_ch 32)
   state_checksums.json  per-tensor (sum, abs-sum) of the reference's freshly
                         constructed G and D state dicts for seed 0 (ctor / RNG parity)
-  small_fwd.pt          seeded inputs and the reference's G / D / DiffAugment / loss outputs
-  small_step.pt         one unmodified train_fns.train step: the 5 returned floats,
+  small_fwd/            seeded inputs and the reference's G / D / DiffAugment / loss outputs
+  small_step/           one unmodified train_fns.train step: the 5 returned floats,
                         per-parameter gradient norms, a few full gradients, u0/sv0 and
                         BN running statistics after the step
   full_checksums.json   ctor checksums of the shipped-size nets (H_base 1 and 3)
+small_fwd/ and small_step/ are golden sets in the layout of golden_io.py.
 """
 import json
 import os
@@ -21,6 +22,9 @@ import sys
 import types
 
 import torch
+
+sys.path.insert(0, os.path.dirname(os.path.abspath(__file__)))
+from golden_io import save_golden  # noqa: E402
 
 REF = "/root/reference"
 HERE = os.path.dirname(os.path.abspath(__file__))
@@ -132,7 +136,7 @@ def main():
         img3 = G3(z3, y)
     out["g3_img_sub"] = img3[:, :, ::4, ::4].clone()
     out["g3_mean_std"] = torch.stack([img3.mean(dim=[1, 2, 3]), img3.std(dim=[1, 2, 3])])
-    torch.save(out, os.path.join(HERE, "small_fwd.pt"))
+    save_golden(os.path.join(HERE, "small_fwd"), out)
 
     # ---------------- one unmodified train step ----------------
     import train_fns
@@ -167,7 +171,7 @@ def main():
                                                     "blocks.5.0.bn3.stored_mean", "blocks.5.0.bn3.stored_var",
                                                     "output_layer.0.stored_var"]}
     step["d_buffers"] = {k: ds[k].clone() for k in ["input_conv.u0", "input_conv.sv0", "embed.u0", "linear1.sv0"]}
-    torch.save(step, os.path.join(HERE, "small_step.pt"))
+    save_golden(os.path.join(HERE, "small_step"), step)
 
     # ---------------- shipped-size ctor checksums ----------------
     full = {}

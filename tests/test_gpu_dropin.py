@@ -2,7 +2,7 @@
 byte under baseline/_ref by tools/fetch_ref.py) drives the B200 modules of iea_gan_b200/dropin -- with the
 reference's own utils.prepare_z_y Distribution tensors, utils.toggle_grad, utils.make_mask, utils.ortho,
 torch's clip_grad_norm_, G.optim / D.optim and utils.apply_ema -- and must reproduce the reference's own CPU run
-of the same step (tests/golden/small_step.pt) or, for two events, the CPU oracle.
+of the same step (the tests/golden/small_step/ golden set) or, for two events, the CPU oracle.
 
 Nothing of the caller is patched: the only hooks are the z_ tensor's sample_() (replaced on the INSTANCE so
 the step sees the golden run's CPU draws) and iea_gan_b200.noise.replay for the in-forward draws.
@@ -29,7 +29,8 @@ def ref_modules():
         pytest.skip("no CUDA device")
     import fetch_ref
     if not fetch_ref.present():
-        pytest.skip("baseline/_ref not staged (python tools/fetch_ref.py in the build container)")
+        pytest.skip("the reference's unmodified train_fns.py / utils/ are not part of this repository: "
+                    "stage them under baseline/_ref with python tools/fetch_ref.py --src <reference checkout>")
     saved_path, saved_mods = list(sys.path), dict(sys.modules)
     fetch_ref.activate(dropin=True)
     import model, train_fns, utils, loss  # noqa: E401

@@ -1,5 +1,5 @@
 """Every module of the drop-in surface, called STAND-ALONE on the B200, against vectors produced by the real
-reference (tests/golden/make_golden_modules.py -> modules.pt): outputs, input gradients, parameter gradients
+reference (tests/golden/make_golden_modules.py -> tests/golden/modules/): outputs, input gradients, parameter gradients
 and the buffers the call leaves behind (u0 / sv0 / running statistics).
 
 Tolerances: fp32 activations (IEA_ACT_DTYPE=fp32, same arithmetic as the reference in another summation
@@ -13,7 +13,6 @@ import pytest
 import torch
 
 pytestmark = pytest.mark.gpu
-GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "modules.pt")
 SN = dict(num_svs=1, num_itrs=1, eps=1e-6)
 
 
@@ -23,10 +22,10 @@ def rel(a, b):
 
 
 @pytest.fixture(scope="module")
-def gold():
+def gold(golden_modules):
     if not torch.cuda.is_available():
         pytest.skip("no CUDA device")
-    return torch.load(GOLDEN)
+    return golden_modules
 
 
 @pytest.fixture(params=["fp32", "bf16"])

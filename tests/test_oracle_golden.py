@@ -27,6 +27,13 @@ def fresh(cfg, seed=0):
     return sg, sd
 
 
+def checksum_close(got, want, abs_sum):
+    """Constructor checksums.  Initialisers that go through the host's BLAS / LAPACK (the QR of the orthogonal init)
+    round differently with the CPU's vector unit and thread count: a tensor's sum moves by up to ~4e-8 of its
+    abs-sum between hosts.  A different draw order or initialiser moves it by ~abs-sum / sqrt(numel) or more."""
+    return abs(got - want) < 1e-9 + 1e-6 * abs_sum
+
+
 def test_ctor_matches_reference_checksums(small_cfg):
     with open(os.path.join(GOLDEN, "state_checksums.json")) as f:
         ref = json.load(f)
@@ -35,8 +42,8 @@ def test_ctor_matches_reference_checksums(small_cfg):
         assert list(s.keys()) == list(ref[name].keys())
         for k, v in s.items():
             assert list(v.shape) == ref[name][k][2], k
-            assert abs(float(v.double().sum()) - ref[name][k][0]) < 1e-9, k
-            assert abs(float(v.double().abs().sum()) - ref[name][k][1]) < 1e-9, k
+            assert checksum_close(float(v.double().sum()), ref[name][k][0], ref[name][k][1]), k
+            assert checksum_close(float(v.double().abs().sum()), ref[name][k][1], ref[name][k][1]), k
 
 
 @pytest.mark.parametrize("hb", [1, 3])
@@ -55,7 +62,7 @@ def test_full_size_ctor_checksums(hb):
         s = net.state_dict()
         assert list(s.keys()) == list(ref[name].keys())
         for k, v in s.items():
-            assert abs(float(v.double().sum()) - ref[name][k][0]) < 1e-9, k
+            assert checksum_close(float(v.double().sum()), ref[name][k][0], ref[name][k][1]), k
 
 
 def test_generator_forward(small_cfg, golden_fwd):
@@ -157,10 +164,10 @@ def test_train_step_matches_unmodified_train_fns(small_cfg, golden_step):
         assert rel(sd[k], v) < 1e-4, k
 
 
-def test_input_pipeline_matches_reference_transforms():
+def test_input_pipeline_matches_reference_transforms(golden_modules):
     """oracle.preprocess_events against the reference's own transform chain (utils/dataloader.py:69-77) run on
     synthetic decoded images by tests/golden/make_golden_modules.py."""
-    d = torch.load(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "modules.pt"))["pipeline"]
+    d = golden_modules["pipeline"]
     got = O.preprocess_events(d["u8"], d["draws"])
     assert got.shape == d["out"].shape == (6, 1, 256, 48)
     assert float((got - d["out"]).abs().max()) < 1e-6

@@ -1,5 +1,5 @@
 import os, sys, torch
-sys.path.insert(0, "/root/repo")
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 def rel(a, b):
     a, b = a.double().cpu(), b.double().cpu()
     return float((a - b).norm() / (b.norm() + 1e-30))

@@ -1,14 +1,15 @@
 """debug: stand-alone GBlock per-parameter errors vs the reference-run vectors; loss trajectories fp32 vs bf16."""
 import functools, json, os, sys
 ROOT = os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
-sys.path.insert(0, ROOT); sys.path.insert(0, os.path.join(ROOT, "tests"))
+sys.path.insert(0, ROOT); sys.path.insert(0, os.path.join(ROOT, "tests")); sys.path.insert(0, os.path.join(ROOT, "tests", "golden"))
 import torch
 os.environ["IEA_ACT_DTYPE"] = "fp32"
 import iea_gan_b200.sn_layers as SL
 from iea_gan_b200 import nets
 import iea_gan_b200 as P
 SN = dict(num_svs=1, num_itrs=1, eps=1e-6)
-gold = torch.load(os.path.join(ROOT, "tests/golden/modules.pt"))
+from golden_io import load_golden
+gold = load_golden(os.path.join(ROOT, "tests/golden/modules"))
 def rel(a, b):
     a, b = a.detach().double().cpu(), b.detach().double().cpu()
     return float((a - b).norm() / (b.norm() + 1e-30))

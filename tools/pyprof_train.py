@@ -1,5 +1,5 @@
 import cProfile, pstats, os, sys, torch
-sys.path.insert(0, "/root/repo")
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import iea_gan_b200 as P
 from iea_gan_b200.default_config import shipped_config
 from iea_gan_b200.train_step import make_train_step, NormalNoise, EMA

@@ -7,6 +7,8 @@ using namespace iea;
 int iea_conv_fprop_generic(const iea_conv_desc* d, cudaStream_t s);
 int iea_conv_fprop_tc(const iea_conv_desc* d, cudaStream_t s);
 int iea_conv_tc_ok(const iea_conv_desc* d);
+int iea_conv_lowres_ok(const iea_conv_desc* d);
+int iea_conv_fprop_lowres(const iea_conv_desc* d, cudaStream_t s);
 int iea_conv_tc2_ok(const iea_conv_desc* d);
 int iea_conv_fprop_tc2(const iea_conv_desc* d, cudaStream_t s);
 int iea_conv_thin_ok(const iea_conv_desc* d);
@@ -17,13 +19,20 @@ int iea_conv_c1_fwd(const iea_conv_desc* d, cudaStream_t s);
 int iea_linear_skinny_ok(const iea_conv_desc* d);
 int iea_linear_skinny(const iea_conv_desc* d, cudaStream_t s);
 
-// tcgen05 variant selection: resident-weights/patch kernel when it applies, else the streaming one.
-// IEA_TC_VARIANT=stream forces the streaming kernel (used by the tests to cover both).
+// tcgen05 variant selection: resident-weights/patch kernel when it applies, then the staged-patch kernel with
+// streamed weights (wide 3x3 layers at low resolution), else the streaming one.
+// IEA_TC_VARIANT=stream forces the streaming kernel (used by the tests to cover both); IEA_LOWRES_TC=0 turns the
+// staged-patch kernel off.  Both kernels tile the pixels alike, so the statistics slots do not depend on the choice.
+static bool lowres_on() {
+  const char* v = getenv("IEA_LOWRES_TC");
+  return !(v && v[0] == '0');
+}
 static int run_tc(const iea_conv_desc* d, cudaStream_t s) {
   const char* v = getenv("IEA_TC_VARIANT");
   const bool force_stream = v && v[0] == 's';
   if (!force_stream && iea_conv_thin_ok(d)) return iea_conv_fprop_thin(d, s);
   if ((!force_stream || !iea_conv_tc_ok(d)) && iea_conv_tc2_ok(d)) return iea_conv_fprop_tc2(d, s);
+  if (!force_stream && lowres_on() && iea_conv_lowres_ok(d)) return iea_conv_fprop_lowres(d, s);
   return iea_conv_fprop_tc(d, s);
 }
 
@@ -50,7 +59,7 @@ extern "C" int iea_conv_stats_slots(const iea_conv_desc* d) {
   if (!iea_conv_tc_ok(d) && !iea_conv_tc2_ok(d)) return tiles;  // generic kernel
   if (!force_stream && iea_conv_thin_ok(d)) return iea_conv_thin_stats_slots(d);
   if ((!force_stream || !iea_conv_tc_ok(d)) && iea_conv_tc2_ok(d)) return iea_conv_tc2_stats_slots(d);
-  return tiles;
+  return tiles;  // conv_tc_kernel and conv_lr_kernel: one slot per 128-pixel tile
 }
 
 extern "C" int iea_conv_tc_supported(const iea_conv_desc* d) { return iea_conv_tc_ok(d) || iea_conv_tc2_ok(d); }

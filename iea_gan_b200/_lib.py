@@ -16,7 +16,7 @@ LIB_PATH = os.path.join(_HERE, "libiea_sm100.so")
 F32, BF16 = 0, 1
 IN_DIRECT, IN_UP2, IN_POOL2 = 0, 1, 2
 ACT_NONE, ACT_RELU, ACT_TANH = 0, 1, 2
-IMPL_AUTO, IMPL_GENERIC, IMPL_TCGEN05 = 0, 1, 2
+IMPL_AUTO, IMPL_GENERIC, IMPL_TCGEN05, IMPL_TC_STREAM = 0, 1, 2, 3
 
 vp, i32, i64, f32 = C.c_void_p, C.c_int32, C.c_int64, C.c_float
 

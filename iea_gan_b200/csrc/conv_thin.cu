@@ -698,7 +698,6 @@ int iea_conv_tc_base_ok(const iea_conv_desc* d, int padded);
 // macro-tile width (in 16x8 / 128-pixel tiles) the kernel uses for this layer; 0: layer not eligible
 static int thin_mt(const iea_conv_desc* d) {
   if (!iea_conv_tc_base_ok(d, d->cout == 1 ? 1 : 0)) return 0;
-  { const char* e_ = getenv("IEA_THIN"); if (e_ && e_[0] == '0') return 0; }  // profiling switch: old kernels only
   // (cout 1 with a 16-row weight pack: the generator's 32->1 output conv; its real channel is stored
   //  straight from the accumulator registers in the storage type of y)
   const bool pad1 = d->cout == 1 && d->cout_tc == 16;
@@ -827,7 +826,6 @@ static int thin_prepare(const iea_conv_desc* d, thin::Params& p, int& grid, uint
   while (stages > 4 && p.stage_off + stages * G::STAGE + tail + tst_bytes > 208 * 1024) stages -= 2;
   p.stages = stages;
   p.depth = stages >= 8 ? 3 : 2;  // items each group keeps in flight (it owns stages/2 slots)
-  { const char* e_ = getenv("IEA_THIN_DEPTH"); if (e_ && atoi(e_) >= 2 && atoi(e_) <= stages / 2) p.depth = atoi(e_); }  // tuning aid
   p.tst_off = (p.stage_off + stages * G::STAGE + 1023) / 1024 * 1024;
   p.res_off = p.tst_off + 2 * 2 * 128 * 64 + 1024;
   p.misc_off = tst ? p.res_off + ring_bytes : p.stage_off + stages * G::STAGE;
@@ -855,12 +853,11 @@ static int thin_launch(const iea_conv_desc* d, cudaStream_t s, int* grid_only) {
   bool tma = TMA_OK && !grid_only && d->in_mode == IEA_IN_DIRECT && d->x_ld % 8 == 0;
   if (tma) { const char* e_ = getenv("IEA_THIN_TMA"); if (e_ && e_[0] == '0') tma = false; }
   if (tma) tma = thin_tensor_map(d, IS3, MT, &tm);
-  // TMA store of the output: the residual flavour of the 1x1 layers, whole sub-tiles only (IEA_THIN_TST=0 disables)
+  // TMA store of the output: the residual flavour of the 1x1 layers, whole sub-tiles only
   alignas(64) CUtensorMap tmy;
   memset(&tmy, 0, sizeof(tmy));
   const bool simple = d->acc_c0 < 0 && d->act == IEA_ACT_NONE && d->cout != 1;
   bool tst = !IS3 && tma && simple && d->res && d->res_mode != IEA_IN_POOL2 && (d->n * (int64_t)d->h * d->w) % (128 * MT) == 0;
-  if (tst) { const char* e_ = getenv("IEA_THIN_TST"); if (e_ && e_[0] == '0') tst = false; }
   alignas(64) CUtensorMap tmr;
   memset(&tmr, 0, sizeof(tmr));
   if (tst) tst = thin_tensor_map_y(d, &tmy) && thin_tensor_map_r(d, &tmr);

@@ -15,7 +15,6 @@
 // m16n8k16 shape matches the 16-channel blocks exactly, ldmatrix takes per-lane row addresses (so the
 // shifted tap views are free) and each g fragment is reused by all 9 taps: ~40 KB of smem reads/tile.
 #include "tc_common.cuh"
-#include <stdlib.h>
 using namespace iea;
 
 namespace wg {
@@ -568,8 +567,23 @@ __global__ void wgrad_reduce_kernel(const float* gpart, int nsplit, int64_t tota
 
 }  // namespace wg
 
-// number of partial slices iea_conv_wgrad_mma will write (0: shape not handled by this kernel)
-static int wgrad_mma_plan(const iea_conv_desc* d, int g_dtype, int g_ld, wg::Params* p, int* npair_out) {
+// The weight-gradient kernel a shape runs on, with its launch geometry.  wgrad_plan() is the one place that
+// chooses it: iea_conv_wgrad_mma_slices sizes gpart from the plan and iea_conv_wgrad_mma launches it.
+struct WgradPlan {
+  enum Kernel { none, c1, tc, macro, mma } kernel = none;
+  int grid = 0;      // per-CTA (tc: per-split) partials, in slices 1..grid of gpart
+  int slices = 0;    // slices of gpart the launch uses; 0: shape not handled (use iea_conv_wgrad)
+  uint32_t smem = 0;
+  wg::P3 p3;                        // macro-tile kernel
+  void (*k3)(wg::P3) = nullptr;
+  wg::Params pm;                    // generic mma.sync kernel
+  void (*km)(wg::Params) = nullptr;
+  int grid_y = 1;
+};
+
+// generic mma.sync kernel: parameters, instance and grid (0: shape not handled by this kernel)
+static int wgrad_mma_plan(const iea_conv_desc* d, int g_dtype, int g_ld, WgradPlan& pl) {
+  wg::Params* p = &pl.pm;
   const bool thin_a = d->cin < 16, thin_g = d->cout < 16;
   if (!thin_a && (d->cin % 16 || d->x_dtype != IEA_BF16 || d->x_ld % 8 || (reinterpret_cast<uintptr_t>(d->x) & 15))) return 0;
   if (thin_a && (d->cin != 1 || d->in_scale || d->in_relu || d->in_mode != IEA_IN_DIRECT)) return 0;
@@ -623,7 +637,18 @@ static int wgrad_mma_plan(const iea_conv_desc* d, int g_dtype, int g_ld, wg::Par
   p->stages = stages;
   p->depth = stages >= 4 ? 3 : 2;
   p->P = P; p->WP = WP;
-  *npair_out = npair;
+  int dev = 0, sms = 148;
+  cudaGetDevice(&dev);
+  cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+  pl.smem = p->stages * p->stage_bytes;
+  const int occ = pl.smem <= 100 * 1024 ? 2 : 1;
+  if (WP > 1 && pl.smem < (uint32_t)(P * (taps * 8 + 4) * 32 * 4)) pl.smem = P * (taps * 8 + 4) * 32 * 4;  // fold scratch
+  pl.grid = p->n_tiles < sms * occ ? p->n_tiles : sms * occ;
+  pl.grid_y = p->gi * (ncb / ncb_l);
+  if (is3) pl.km = npair == 1 ? wg::wgrad_mma_kernel<9, 1> : npair == 2 ? wg::wgrad_mma_kernel<9, 2> : nullptr;
+  else pl.km = npair == 1 ? wg::wgrad_mma_kernel<1, 1> : npair == 2 ? wg::wgrad_mma_kernel<1, 2>
+             : npair == 4 ? wg::wgrad_mma_kernel<1, 4> : npair == 8 ? wg::wgrad_mma_kernel<1, 8>
+             : npair == 16 ? wg::wgrad_mma_kernel<1, 16> : nullptr;
   return 1;
 }
 
@@ -632,7 +657,6 @@ int iea_conv_c1_wgrad(const iea_conv_desc* d, const void* g, int g_dtype, int g_
 
 // macro-tile kernel: 0 = shape not handled, else MT (sub-tiles per macro tile)
 static int wgrad3_mt(const iea_conv_desc* d, int g_dtype, int g_ld) {
-  { const char* e_ = getenv("IEA_WGRAD3"); if (e_ && e_[0] == '0') return 0; }  // test / profiling switch: generic mma kernel
   const bool is3 = d->ksize == 3;
   if (is3) {
     if ((d->cin != 16 && d->cin != 32) || (d->cout != 16 && d->cout != 32)) return 0;
@@ -679,125 +703,91 @@ static int wgrad3_setup(const iea_conv_desc* d, wg::P3& p, int& grid, uint32_t& 
   grid = p.n_macro < sms * occ ? p.n_macro : sms * occ;
   return 0;
 }
-// grid of the macro-tile launch (0: not handled); launches when parts != nullptr
-static int wgrad3_run(const iea_conv_desc* d, const void* g, int g_dtype, int g_ld, float* parts, float* cs_parts, cudaStream_t s) {
+// macro-tile kernel: instance, parameters and grid (false: shape not handled by this kernel)
+static bool wgrad3_plan(const iea_conv_desc* d, int g_dtype, int g_ld, WgradPlan& pl) {
   const int mt = wgrad3_mt(d, g_dtype, g_ld);
-  if (!mt) return 0;
-  wg::P3 p; int grid = 0; uint32_t smem = 0;
+  if (!mt) return false;
   const int cpa = d->cin / 8, cpg = d->cout / 8;
   const bool is3 = d->ksize == 3;
-  p.g = (const bf16*)g; p.g_ld = g_ld; p.gpart = parts; p.cs_parts = cs_parts;
-#define IEA_W3(A_, G_, M_, I_)                                                                                     \
-  if (cpa == A_ && cpg == G_ && mt == M_ && is3 == I_) {                                                                     \
-    wgrad3_setup<A_, G_, M_, I_>(d, p, grid, smem);                                                                 \
-    if (parts) {                                                                                                  \
-      auto kern = wg::wgrad3_kernel<A_, G_, M_, I_>;                                                                \
-      if (cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess) return -1; \
-      kern<<<grid, 256, smem, s>>>(p);                                                                            \
-    }                                                                                                             \
-    return grid;                                                                                                  \
+#define IEA_W3(A_, G_, M_, I_)                                  \
+  if (cpa == A_ && cpg == G_ && mt == M_ && is3 == I_) {        \
+    wgrad3_setup<A_, G_, M_, I_>(d, pl.p3, pl.grid, pl.smem);   \
+    pl.k3 = wg::wgrad3_kernel<A_, G_, M_, I_>;                  \
+    return true;                                                \
   }
   IEA_W3(2, 2, 4, true) IEA_W3(2, 2, 2, true) IEA_W3(2, 4, 2, true) IEA_W3(4, 2, 2, true) IEA_W3(4, 4, 2, true)
   IEA_W3(2, 2, 4, false) IEA_W3(2, 2, 2, false) IEA_W3(2, 2, 1, false) IEA_W3(2, 4, 2, false) IEA_W3(2, 4, 1, false)
   IEA_W3(4, 2, 2, false) IEA_W3(4, 2, 1, false) IEA_W3(4, 4, 2, false) IEA_W3(4, 4, 1, false) IEA_W3(2, 8, 1, false)
   IEA_W3(8, 2, 1, false) IEA_W3(4, 8, 1, false) IEA_W3(8, 4, 1, false)
 #undef IEA_W3
-  return 0;
+  return false;
 }
 
 int iea_conv_wgrad_tc_splits(const iea_conv_desc* d, int g_dtype, int g_ld);
 int iea_conv_wgrad_tc(const iea_conv_desc* d, const void* g, int g_dtype, int g_ld, float* gpart, cudaStream_t s);
-// wide low-resolution layers: TMEM-accumulating tcgen05 kernel (conv_wgrad_tc.cu); IEA_WGRAD_TC=0 switches it off
-static int wgrad_tc_splits(const iea_conv_desc* d, int g_dtype, int g_ld) {
-  static const int on = [] { const char* v = getenv("IEA_WGRAD_TC"); return !(v && v[0] == '0'); }();
-  return on ? iea_conv_wgrad_tc_splits(d, g_dtype, g_ld) : 0;
+
+// first kernel that takes the shape: the 1-channel side (conv_c1.cu), the TMEM-accumulating tcgen05 kernel of the
+// wide low-resolution layers (conv_wgrad_tc.cu), the macro-tile kernel, the generic mma.sync kernel
+static WgradPlan wgrad_plan(const iea_conv_desc* d, int g_dtype, int g_ld) {
+  WgradPlan pl;
+  if ((pl.grid = iea_conv_c1_wgrad_grid(d, g_dtype, g_ld))) pl.kernel = WgradPlan::c1;
+  else if ((pl.grid = iea_conv_wgrad_tc_splits(d, g_dtype, g_ld))) pl.kernel = WgradPlan::tc;
+  else if (wgrad3_plan(d, g_dtype, g_ld, pl)) pl.kernel = WgradPlan::macro;
+  else if (wgrad_mma_plan(d, g_dtype, g_ld, pl)) pl.kernel = WgradPlan::mma;
+  else return pl;
+  // the per-CTA partials + one slot for their sum (slice 0 after the call); the mma.sync kernels also need room
+  // for their per-CTA column sums of g (grid * cout floats) behind them
+  pl.slices = pl.grid + 1;
+  if (pl.kernel == WgradPlan::macro || pl.kernel == WgradPlan::mma) {
+    const int64_t total = (int64_t)d->cout * d->ksize * d->ksize * d->cin;
+    pl.slices += (int)(((int64_t)pl.grid * d->cout + total - 1) / total);
+  }
+  return pl;
 }
 
 extern "C" int iea_conv_wgrad_mma_slices(const iea_conv_desc* d, int g_dtype, int g_ld) {
-  if (const int c1g = iea_conv_c1_wgrad_grid(d, g_dtype, g_ld)) return c1g + 1;  // 1-channel side: conv_c1.cu
-  if (const int st = wgrad_tc_splits(d, g_dtype, g_ld)) return st + 1;
-  if (const int g3 = wgrad3_run(d, nullptr, g_dtype, g_ld, nullptr, nullptr, nullptr)) {
-    const int64_t total = (int64_t)d->cout * d->ksize * d->ksize * d->cin;
-    return g3 + 1 + (int)(((int64_t)g3 * d->cout + total - 1) / total);
-  }
-  wg::Params p; int npair;
-  if (!wgrad_mma_plan(d, g_dtype, g_ld, &p, &npair)) return 0;
-  int dev = 0, sms = 148;
-  cudaGetDevice(&dev);
-  cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-  const int occ = p.stages * p.stage_bytes <= 100 * 1024 ? 2 : 1;
-  const int grid = p.n_tiles < sms * occ ? p.n_tiles : sms * occ;
-  // grid per-CTA partials + one slot for their sum (slice 0 after the call) + room for the per-CTA
-  // column sums of g (grid * cout floats) behind them
-  const int64_t total = (int64_t)d->cout * d->ksize * d->ksize * d->cin;
-  return grid + 1 + (int)(((int64_t)grid * d->cout + total - 1) / total);
+  return wgrad_plan(d, g_dtype, g_ld).slices;
 }
 
 extern "C" int iea_conv_wgrad_mma(const iea_conv_desc* d, const void* g, int g_dtype, int g_ld, float* gpart,
                                   float* dbias, iea_stream_t stream) {
-  if (const int c1g = iea_conv_c1_wgrad_grid(d, g_dtype, g_ld)) {
-    const int64_t total = (int64_t)d->cout * 9 * d->cin;
-    int rc = iea_conv_c1_wgrad(d, g, g_dtype, g_ld, gpart + total, (cudaStream_t)stream);
-    if (rc) return rc;
-    int rb = (int)((total + 255) / 256);
-    wg::wgrad_reduce_kernel<<<rb, 256, 0, (cudaStream_t)stream>>>(gpart + total, c1g, total, gpart);
-    return check_launch("iea_conv_wgrad_mma(1-channel)");  // 0: the bias gradient was not produced
-  }
-  if (wgrad_tc_splits(d, g_dtype, g_ld))  // (0: the bias gradient is not produced by this path)
-    return iea_conv_wgrad_tc(d, g, g_dtype, g_ld, gpart, (cudaStream_t)stream);
-  if (const int g3 = wgrad3_run(d, nullptr, g_dtype, g_ld, nullptr, nullptr, nullptr)) {  // macro-tile kernel
-    const int64_t total = (int64_t)d->cout * d->ksize * d->ksize * d->cin;
-    float* parts = gpart + total;
-    float* csp = dbias ? gpart + (int64_t)(g3 + 1) * total : nullptr;
-    const int rc3 = wgrad3_run(d, g, g_dtype, g_ld, parts, csp, (cudaStream_t)stream);
-    IEA_CHECK_ARG(rc3 == g3, "iea_conv_wgrad_mma(macro tile): launch set-up failed");
-    int rb = (int)((total + 255) / 256);
-    wg::wgrad_reduce_kernel<<<rb, 256, 0, (cudaStream_t)stream>>>(parts, g3, total, gpart);
-    if (dbias) wg::wgrad_reduce_kernel<<<(d->cout + 255) / 256, 256, 0, (cudaStream_t)stream>>>(csp, g3, d->cout, dbias);
-    const int rc = check_launch("iea_conv_wgrad_mma(macro tile)");
-    return rc ? rc : (dbias ? 1 : 0);
-  }
-  wg::Params p; int npair;
-  IEA_CHECK_ARG(wgrad_mma_plan(d, g_dtype, g_ld, &p, &npair), "iea_conv_wgrad_mma: shape not handled (cin=%d cout=%d k=%d)",
-                d->cin, d->cout, d->ksize);
-  p.g = g; p.g_dtype = g_dtype; p.g_ld = g_ld; p.gpart = gpart;
-  int dev = 0, sms = 148;
-  cudaGetDevice(&dev);
-  cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-  const int taps_ = d->ksize * d->ksize;
-  const int nib_ = p.cin_eff / 16, ncb_ = p.cout_eff / 16;
-  uint32_t smem = p.stages * p.stage_bytes;
-  const int occ = smem <= 100 * 1024 ? 2 : 1;
-  if (p.WP > 1 && smem < (uint32_t)(p.P * (taps_ * 8 + 4) * 32 * 4)) smem = p.P * (taps_ * 8 + 4) * 32 * 4;  // fold scratch
-  const int grid = p.n_tiles < sms * occ ? p.n_tiles : sms * occ;
+  WgradPlan pl = wgrad_plan(d, g_dtype, g_ld);
+  IEA_CHECK_ARG(pl.kernel != WgradPlan::none, "iea_conv_wgrad_mma: shape not handled (cin=%d cout=%d k=%d)", d->cin,
+                d->cout, d->ksize);
   cudaStream_t s = (cudaStream_t)stream;
-  const int64_t total = (int64_t)d->cout * taps_ * d->cin;
+  const int64_t total = (int64_t)d->cout * d->ksize * d->ksize * d->cin;
   float* parts = gpart + total;  // slices 1..grid hold the per-CTA partials, slice 0 receives their sum
-  p.gpart = parts;
-  p.cs_parts = dbias ? gpart + (int64_t)(grid + 1) * total : nullptr;
-  auto launch = [&](auto kern) -> int {
-    IEA_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    kern<<<dim3(grid, (nib_ / p.nib_l) * (ncb_ / p.ncb_l)), 256, smem, s>>>(p);
-    return 0;
-  };
-  int rc = -2;
-  const bool is3 = d->ksize == 3;
-  if (is3) {
-    if (npair == 1) rc = launch(wg::wgrad_mma_kernel<9, 1>);
-    else if (npair == 2) rc = launch(wg::wgrad_mma_kernel<9, 2>);
-  } else {
-    if (npair == 1) rc = launch(wg::wgrad_mma_kernel<1, 1>);
-    else if (npair == 2) rc = launch(wg::wgrad_mma_kernel<1, 2>);
-    else if (npair == 4) rc = launch(wg::wgrad_mma_kernel<1, 4>);
-    else if (npair == 8) rc = launch(wg::wgrad_mma_kernel<1, 8>);
-    else if (npair == 16) rc = launch(wg::wgrad_mma_kernel<1, 16>);
-  }
-  IEA_CHECK_ARG(rc != -2, "iea_conv_wgrad_mma: no kernel instance for %d block pairs per warp", npair);
-  if (rc) return rc;
+  float* cs_parts = dbias ? gpart + (int64_t)(pl.grid + 1) * total : nullptr;
   int rb = (int)((total + 255) / 256);
-  if (rb > 592) rb = 592;
-  wg::wgrad_reduce_kernel<<<rb, 256, 0, s>>>(parts, grid, total, gpart);
-  if (dbias) wg::wgrad_reduce_kernel<<<(d->cout + 255) / 256, 256, 0, s>>>(p.cs_parts, grid, d->cout, dbias);
-  rc = check_launch("iea_conv_wgrad_mma");
-  return rc ? rc : (dbias ? 1 : 0);  // 1: dbias holds the column sums of g
+  const char* what = "iea_conv_wgrad_mma";
+  switch (pl.kernel) {
+    case WgradPlan::none: break;
+    case WgradPlan::tc:  // (0: the bias gradient is not produced by this path)
+      return iea_conv_wgrad_tc(d, g, g_dtype, g_ld, gpart, s);
+    case WgradPlan::c1: {
+      const int rc = iea_conv_c1_wgrad(d, g, g_dtype, g_ld, parts, s);
+      if (rc) return rc;
+      cs_parts = nullptr;  // (the bias gradient is not produced by this path)
+      what = "iea_conv_wgrad_mma(1-channel)";
+      break;
+    }
+    case WgradPlan::macro:
+      pl.p3.g = (const bf16*)g; pl.p3.g_ld = g_ld; pl.p3.gpart = parts; pl.p3.cs_parts = cs_parts;
+      IEA_CHECK_ARG(cudaFuncSetAttribute(pl.k3, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)pl.smem) == cudaSuccess,
+                    "iea_conv_wgrad_mma(macro tile): launch set-up failed");
+      pl.k3<<<pl.grid, 256, pl.smem, s>>>(pl.p3);
+      what = "iea_conv_wgrad_mma(macro tile)";
+      break;
+    case WgradPlan::mma:
+      IEA_CHECK_ARG(pl.km, "iea_conv_wgrad_mma: no kernel instance for %d block pairs", pl.pm.P);
+      pl.pm.g = g; pl.pm.g_dtype = g_dtype; pl.pm.g_ld = g_ld; pl.pm.gpart = parts; pl.pm.cs_parts = cs_parts;
+      IEA_CUDA(cudaFuncSetAttribute(pl.km, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)pl.smem));
+      pl.km<<<dim3(pl.grid, pl.grid_y), 256, pl.smem, s>>>(pl.pm);
+      if (rb > 592) rb = 592;
+      break;
+  }
+  wg::wgrad_reduce_kernel<<<rb, 256, 0, s>>>(parts, pl.grid, total, gpart);
+  if (cs_parts) wg::wgrad_reduce_kernel<<<(d->cout + 255) / 256, 256, 0, s>>>(cs_parts, pl.grid, d->cout, dbias);
+  const int rc = check_launch(what);
+  return rc ? rc : (cs_parts ? 1 : 0);  // 1: dbias holds the column sums of g
 }

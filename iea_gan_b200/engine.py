@@ -44,7 +44,7 @@ def act_dtype():
 
 
 def conv_impl():
-    return {"auto": L.IMPL_AUTO, "generic": L.IMPL_GENERIC, "tcgen05": L.IMPL_TCGEN05}[
+    return {"auto": L.IMPL_AUTO, "generic": L.IMPL_GENERIC, "tcgen05": L.IMPL_TCGEN05, "stream": L.IMPL_TC_STREAM}[
         _env(b"IEA_CONV_IMPL", "IEA_CONV_IMPL", "auto")]
 
 
@@ -599,7 +599,7 @@ def conv(tape, xv, layer, n, h, w, k, *, bias=None, in_mode=L.IN_DIRECT, in_relu
         if (k == 1 and in_mode == L.IN_DIRECT and grouped is None and act == L.ACT_NONE and wd_tc is not None
                 and yv.g.dtype == torch.bfloat16 and xv.t.dtype == torch.bfloat16 and y.dtype == torch.bfloat16
                 and conv_impl() != L.IMPL_GENERIC and (xv.need or ss is not None or wls[0].weight.requires_grad)
-                and (res is None or dt(res.t) == L.BF16) and _env(b"IEA_BWD1X1", "IEA_BWD1X1", "1") != "0"):
+                and (res is None or dt(res.t) == L.BF16)):
             dfq = fwd_desc()
             grid = call("iea_conv_bwd1x1_grid", C.byref(dfq))
             if grid > 0:

@@ -28,7 +28,11 @@ typedef void* iea_stream_t; /* cudaStream_t */
 enum iea_dtype { IEA_F32 = 0, IEA_BF16 = 1 };
 enum iea_in_mode { IEA_IN_DIRECT = 0, IEA_IN_UP2 = 1, IEA_IN_POOL2 = 2 };
 enum iea_act { IEA_ACT_NONE = 0, IEA_ACT_RELU = 1, IEA_ACT_TANH = 2 };
-enum iea_impl { IEA_IMPL_AUTO = 0, IEA_IMPL_GENERIC = 1, IEA_IMPL_TCGEN05 = 2 };
+/* convolution kernel choice (iea_conv_desc.impl): AUTO picks by shape; GENERIC forces the CUDA-core kernel;
+ * TCGEN05 forces the tcgen05 kernels (an error where they reject the shape); TC_STREAM is TCGEN05 with the
+ * streaming conv_tc kernel wherever it accepts the shape (the reference the other tcgen05 kernels are checked
+ * against), else the resident-weight conv_tc2 kernel. */
+enum iea_impl { IEA_IMPL_AUTO = 0, IEA_IMPL_GENERIC = 1, IEA_IMPL_TCGEN05 = 2, IEA_IMPL_TC_STREAM = 3 };
 
 /* ---- library ------------------------------------------------------------------ */
 int iea_version(void);
@@ -116,7 +120,8 @@ typedef struct {
 int iea_conv_fprop(const iea_conv_desc* d /* host */, iea_stream_t stream);
 /* number of batch-norm partial-sum slots PER EVENT that iea_conv_fprop writes into d->stats for this
  * descriptor (d->stats must be non-NULL when asking): the buffer is [events][slots][cout][2] floats and
- * must be zero-filled by the caller; 0 = the kernel cannot emit statistics for this geometry. */
+ * must be zero-filled by the caller; 0 = the kernel cannot emit statistics for this geometry.  The count
+ * comes from the same kernel choice iea_conv_fprop makes, d->impl included. */
 int iea_conv_stats_slots(const iea_conv_desc* d /* host */);
 /* 1 if the tcgen05 path accepts this descriptor */
 int iea_conv_tc_supported(const iea_conv_desc* d /* host */);

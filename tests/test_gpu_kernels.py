@@ -268,7 +268,7 @@ def _tc_vs_generic(eng, variant, cin, cout, k, mode, relu, aff, resm, hw, n):
     (<= 1 ulp of bf16 = 2^-8 relative per element; 6e-3 relative L2 bound) -- forward, statistics
     and every backward product that runs through the kernel (data gradient)."""
     os.environ["IEA_ACT_DTYPE"] = "bf16"
-    os.environ["IEA_TC_VARIANT"] = variant
+    tc_impl = "stream" if variant == "stream" else "tcgen05"  # stream: conv_tc_kernel wherever it takes the shape
     try:
         dev = "cuda"
         torch.manual_seed(5)
@@ -288,7 +288,7 @@ def _tc_vs_generic(eng, variant, cin, cout, k, mode, relu, aff, resm, hw, n):
             rh, rw = (h // 2, w // 2) if resm == 1 else ((2 * h, 2 * w) if resm == 2 else (h, w))
             res = torch.randn(n, rh, rw, cout + 16, device=dev).bfloat16()
         outs = {}
-        for impl in ("generic", "tcgen05"):
+        for impl in ("generic", tc_impl):
             os.environ["IEA_CONV_IMPL"] = impl
             tape = eng.Tape(True)
             xv = eng.Var(x)
@@ -304,7 +304,7 @@ def _tc_vs_generic(eng, variant, cin, cout, k, mode, relu, aff, resm, hw, n):
             # statistics: compare per-event totals (the two kernels tile the image differently)
             st = yv.bn[0].reshape(n // 40, yv.bn[1], cout, 2).sum(1) if yv.bn else None
             outs[impl] = (yv.t.float(), st, xv.g.float(), tape.pgrads[id(m.weight)].clone())
-        a, b = outs["generic"], outs["tcgen05"]
+        a, b = outs["generic"], outs[tc_impl]
         assert rel(b[0], a[0]) < 6e-3
         if a[1] is not None:
             assert rel(b[1], a[1]) < 6e-3
@@ -313,7 +313,6 @@ def _tc_vs_generic(eng, variant, cin, cout, k, mode, relu, aff, resm, hw, n):
     finally:
         os.environ.pop("IEA_ACT_DTYPE", None)
         os.environ.pop("IEA_CONV_IMPL", None)
-        os.environ.pop("IEA_TC_VARIANT", None)
 
 
 @pytest.mark.parametrize("cin,cout,k,hw,gdt", [(1, 32, 3, (32, 32), "bf16"), (32, 1, 3, (32, 32), "fp32"),

@@ -1,5 +1,5 @@
 """The staged-patch tcgen05 kernel of the wide low-resolution 3x3 layers (conv_lr_kernel in conv_tc.cu) against the
-streaming kernel (conv_tc_kernel, IEA_TC_VARIANT=stream) on the same descriptor.  Both accumulate every output
+streaming kernel (conv_tc_kernel, IEA_CONV_IMPL=stream) on the same descriptor.  Both accumulate every output
 element over the same products in the same order (tap, k block, 16-channel step) and tile the pixels alike, so
 the layer output, its batch-norm partial sums and the data gradient must be bitwise equal.  Shapes the new kernel
 does not take must fall back to the streaming kernel; the profiler's kernel names show which one ran."""
@@ -13,6 +13,7 @@ from test_gpu_kernels import _tc_vs_generic, make_sn_conv
 pytestmark = pytest.mark.gpu
 
 NEW, OLD = "conv_lr_kernel", "conv_tc_kernel"
+STREAM = {"IEA_CONV_IMPL": "stream"}  # the streaming kernel wherever it takes the shape
 
 
 @pytest.fixture(scope="module")
@@ -63,7 +64,7 @@ def _run(eng, variant, cin, cout, mode, relu, aff, resm, hw, n, stats):
         st = yv.bn[0].clone() if (stats and yv.bn) else None
         return (yv.t.clone(), st, xv.g.clone()), names
     finally:
-        for k in ("IEA_ACT_DTYPE", "IEA_TC_VARIANT", "IEA_LOWRES_TC"):
+        for k in ("IEA_ACT_DTYPE", "IEA_CONV_IMPL"):
             os.environ.pop(k, None)
 
 
@@ -93,9 +94,9 @@ CASES = [
 
 
 @pytest.mark.parametrize("cin,cout,mode,relu,aff,resm,hw,n", CASES)
-def test_lowres_matches_stream_bitwise(eng, cin, cout, mode, relu, aff, resm, hw, n):
+def test_lowres_matches_stream_impl_bitwise(eng, cin, cout, mode, relu, aff, resm, hw, n):
     new, kn = _run(eng, {}, cin, cout, mode, relu, aff, resm, hw, n, True)
-    old, ko = _run(eng, {"IEA_TC_VARIANT": "stream"}, cin, cout, mode, relu, aff, resm, hw, n, True)
+    old, ko = _run(eng, STREAM, cin, cout, mode, relu, aff, resm, hw, n, True)
     assert NEW in kn, "the staged-patch kernel did not run: " + kn
     assert NEW not in ko and OLD in ko
     for what, a, b in zip(("y", "statistics", "dx"), new, old):
@@ -111,15 +112,9 @@ def test_lowres_partial_last_tile(eng, hw, n):
     """An odd image count at 8x8, where a 128-pixel tile holds two images: the last tile's second image does not
     exist and its rows must read as zero padding (no statistics: they need whole events)."""
     new, kn = _run(eng, {}, 128, 128, 0, True, True, None, hw, n, False)
-    old, _ = _run(eng, {"IEA_TC_VARIANT": "stream"}, 128, 128, 0, True, True, None, hw, n, False)
+    old, _ = _run(eng, STREAM, 128, 128, 0, True, True, None, hw, n, False)
     assert NEW in kn
     assert _same(new[0], old[0]) and _same(new[2], old[2])
-
-
-def test_lowres_switch_off(eng):
-    """IEA_LOWRES_TC=0 keeps these layers on the streaming kernel."""
-    _, k = _run(eng, {"IEA_LOWRES_TC": "0"}, 128, 128, 1, True, True, None, (16, 16), 40, True)
-    assert NEW not in k and OLD in k
 
 
 # the H_base = 3 widths (4x12, 8x24, 16x48) and 4x4 stay on the streaming kernel
@@ -127,7 +122,7 @@ def test_lowres_switch_off(eng):
                                      ((4, 4), 1)])
 def test_lowres_fallback_shapes(eng, hw, mode):
     new, kn = _run(eng, {}, 128, 128, mode, True, True, 0, hw, 40, True)
-    old, _ = _run(eng, {"IEA_TC_VARIANT": "stream"}, 128, 128, mode, True, True, 0, hw, 40, True)
+    old, _ = _run(eng, STREAM, 128, 128, mode, True, True, 0, hw, 40, True)
     assert NEW not in kn and OLD in kn
     for a, b in zip(new, old):
         assert _same(a, b)

@@ -1,5 +1,6 @@
 """Per-launch timing of the wide low-resolution convolutions of one Generator sampling pass (H_base 1), streaming
-kernel (IEA_LOWRES_TC=0) against the staged-patch kernel (IEA_LOWRES_TC=1) in the same process.
+kernel (the descriptor's impl set to IMPL_TC_STREAM) against the default choice, the staged-patch kernel where it
+takes the shape, in the same process.
 
 The descriptors are captured from a real sampling pass of `events` x 40 images; each one is then launched on its
 own, old and new alternating, with CUDA events around every launch.  A layer's inputs (<= 42 MB) stay in the
@@ -73,27 +74,28 @@ def main():
     torch.cuda.synchronize()
     stream = L.stream()
 
-    def launch(d, on):
-        os.environ["IEA_LOWRES_TC"] = "1" if on else "0"
-        E_.call("iea_conv_fprop", C.byref(d), stream)
+    def streaming(d):
+        d = L.ConvDesc.from_buffer_copy(d)
+        d.impl = L.IMPL_TC_STREAM
+        return d
+    arms = [(streaming(d), d) for d in descs]  # (old: streaming kernel, new: as captured)
 
     times = [([], []) for _ in descs]
     ev = [[(torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)) for _ in range(2)]
           for _ in descs]
     for rep in range(reps + 5):  # 5 warm-up rounds
         pending = []
-        for i, d in enumerate(descs):
+        for i, arm in enumerate(arms):
             for on in (0, 1) if rep % 2 == 0 else (1, 0):
                 a, b = ev[i][on]
                 a.record()
-                launch(d, on)
+                E_.call("iea_conv_fprop", C.byref(arm[on]), stream)
                 b.record()
                 pending.append((i, on, a, b))
         torch.cuda.synchronize()
         if rep >= 5:
             for i, on, a, b in pending:
                 times[i][on].append(a.elapsed_time(b))
-    os.environ.pop("IEA_LOWRES_TC", None)
 
     print("# %s" % gpu_info())
     print("# Generator sampling, H_base 1, %d events (%d images): %d wide low-resolution launches, median of %d "

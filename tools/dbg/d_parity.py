@@ -1,5 +1,5 @@
-"""Relative errors of the full-size Discriminator (bf16) against the fp32 CPU oracle: default engine, the opt-in
-pooled-once shortcut (IEA_DBLOCK_POOL_ONCE=1), and the latter without the fused 1x1 backward."""
+"""Relative errors of the full-size Discriminator (bf16) against the fp32 CPU oracle: default engine and the opt-in
+pooled-once shortcut (IEA_DBLOCK_POOL_ONCE=1)."""
 import os, sys, torch
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__)))))
 import iea_gan_b200 as P
@@ -27,7 +27,7 @@ xr = x.clone().requires_grad_(True)
 pr, er, orr = O.discriminator_forward(sd, dict(cfg, device="cpu"), xr, y, training=True)
 ((orr * go).sum() + (er * ge).sum()).backward()
 res = {}
-for tag, env in (("once", {"IEA_DBLOCK_POOL_ONCE": "1"}), ("old", {}), ("once_nofuse", {"IEA_DBLOCK_POOL_ONCE": "1", "IEA_BWD1X1": "0"})):
+for tag, env in (("once", {"IEA_DBLOCK_POOL_ONCE": "1"}), ("old", {})):
     os.environ.update(env)
     torch.manual_seed(0)
     D = P.Discriminator(**cfg)
@@ -42,6 +42,6 @@ for tag, env in (("once", {"IEA_DBLOCK_POOL_ONCE": "1"}), ("old", {}), ("once_no
     got = dict(D.named_parameters())
     res[tag] = {"e": rel(e, er), "o": rel(o, orr), "dx": rel(xg.grad, xr.grad)}
     res[tag].update({n: rel(got[n].grad, sd[n].grad) for n in names})
-print("%-34s %10s %10s %10s" % ("", "pool_once", "default", "once_nofuse"))
+print("%-34s %10s %10s" % ("", "pool_once", "default"))
 for k in res["once"]:
-    print("%-34s %10.4f %10.4f %10.4f" % (k, res["once"][k], res["old"][k], res["once_nofuse"][k]))
+    print("%-34s %10.4f %10.4f" % (k, res["once"][k], res["old"][k]))

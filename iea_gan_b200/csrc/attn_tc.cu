@@ -34,16 +34,9 @@ constexpr int CKC = CK / 8, CVC = CV / 8;          // 16-byte chunks per row
 constexpr uint32_t PL = BLK * 16 + 16;             // plane pitch (16-byte skew: conflict-free staging)
 constexpr float LOG2E = 1.4426950408889634f;
 
-__host__ __device__ constexpr uint32_t idesc(int n, bool a_mn, bool b_mn) {
-  return (1u << 4) | (1u << 7) | (1u << 10) | ((a_mn ? 1u : 0u) << 15) | ((b_mn ? 1u : 0u) << 16) |
-         ((uint32_t)(n >> 3) << 17) | ((uint32_t)(128 >> 4) << 24);
-}
 __device__ __forceinline__ uint64_t desc_k(uint32_t addr) { return make_desc(addr, PL, 128); }    // K-major
 __device__ __forceinline__ uint64_t desc_mn(uint32_t addr) { return make_desc(addr, 128, PL); }   // MN-major
 
-__device__ __forceinline__ void cp16(uint32_t dst, const void* src) {
-  asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(dst), "l"(src) : "memory");
-}
 // 128 rows of CH 16-byte chunks (row pitch ld elements) -> planes
 template <int CH>
 __device__ __forceinline__ void stage(uint32_t dst, const bf16* src, int ld) {
@@ -54,8 +47,8 @@ __device__ __forceinline__ void stage(uint32_t dst, const bf16* src, int ld) {
   }
 }
 __device__ __forceinline__ void staged_ready() {
-  asm volatile("cp.async.commit_group;" ::: "memory");
-  asm volatile("cp.async.wait_group 0;" ::: "memory");
+  cp_async_commit();
+  cp_async_wait<0>();
   fence_async_smem();
   tc_fence_before();
   __syncthreads();
@@ -70,13 +63,6 @@ __device__ __forceinline__ void mma_kk(uint32_t tacc, uint32_t a, uint32_t b, in
 __device__ __forceinline__ void mma_kmn(uint32_t tacc, uint32_t a, uint32_t b, int n, bool acc) {
 #pragma unroll
   for (int j = 0; j < BLK / 16; ++j) tc_mma(tacc, desc_k(a + 2 * j * PL), desc_mn(b + j * 256), idesc(n, false, true), (acc || j > 0) ? 1u : 0u);
-}
-__device__ __forceinline__ void tmem_alloc(uint32_t slot, uint32_t cols) {
-  asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(slot), "r"(cols));
-  asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;");
-}
-__device__ __forceinline__ void tmem_free(uint32_t base, uint32_t cols) {
-  asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(base), "r"(cols));
 }
 __device__ __forceinline__ void st16(uint32_t addr, const uint4& q) {
   asm volatile("st.shared.v4.b32 [%0], {%1,%2,%3,%4};" ::"r"(addr), "r"(q.x), "r"(q.y), "r"(q.z), "r"(q.w) : "memory");
@@ -97,7 +83,7 @@ __device__ __forceinline__ Ctx setup(uint8_t* smem, uint32_t bar_off, uint32_t c
   uint32_t* slot = reinterpret_cast<uint32_t*>(smem + bar_off + 8);
   if (threadIdx.x == 0) {
     mbar_init(c.bar, 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    fence_mbar_init();
   }
   if (threadIdx.x < 32) tmem_alloc(smem_u32(slot), cols);
   tc_fence_before();

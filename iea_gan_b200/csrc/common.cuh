@@ -89,6 +89,65 @@ __device__ __forceinline__ float block_max(float v, float* red) {
   return red[32];
 }
 
+// packed fp32 pairs (Blackwell FFMA2 / FADD2): half the issue slots of scalar fp32
+__device__ __forceinline__ float2 ffma2(float2 a, float2 b, float2 c) {
+  float2 r;
+  asm("fma.rn.f32x2 %0, %1, %2, %3;" : "=l"(reinterpret_cast<unsigned long long&>(r))
+      : "l"(reinterpret_cast<unsigned long long&>(a)), "l"(reinterpret_cast<unsigned long long&>(b)),
+        "l"(reinterpret_cast<unsigned long long&>(c)));
+  return r;
+}
+__device__ __forceinline__ float2 fadd2(float2 a, float2 b) {
+  float2 r;
+  asm("add.rn.f32x2 %0, %1, %2;" : "=l"(reinterpret_cast<unsigned long long&>(r))
+      : "l"(reinterpret_cast<unsigned long long&>(a)), "l"(reinterpret_cast<unsigned long long&>(b)));
+  return r;
+}
+
+// bf16 <-> fp32: two channels in a 32-bit word, eight in a 16-byte chunk
+__device__ __forceinline__ float2 bf2_to_f2(uint32_t w) { return make_float2(__uint_as_float(w << 16), __uint_as_float(w & 0xFFFF0000u)); }
+__device__ __forceinline__ uint32_t pack2(float a, float b) {
+  __nv_bfloat162 t = __floats2bfloat162_rn(a, b);
+  return *reinterpret_cast<uint32_t*>(&t);
+}
+__device__ __forceinline__ void unpack8(const uint4& q, float* f) {
+  const uint32_t w[4] = {q.x, q.y, q.z, q.w};
+#pragma unroll
+  for (int i = 0; i < 4; ++i) {
+    f[2 * i] = __uint_as_float(w[i] << 16);
+    f[2 * i + 1] = __uint_as_float(w[i] & 0xFFFF0000u);
+  }
+}
+__device__ __forceinline__ uint4 pack8(const float* f) {
+  return make_uint4(pack2(f[0], f[1]), pack2(f[2], f[3]), pack2(f[4], f[5]), pack2(f[6], f[7]));
+}
+
+// 16-byte global -> shared copy (cp.async.cg) and its commit / wait groups
+__device__ __forceinline__ void cp16(uint32_t dst, const void* src) {
+  asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(dst), "l"(src) : "memory");
+}
+__device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
+template <int N>  // wait until at most N committed groups are still in flight
+__device__ __forceinline__ void cp_async_wait() { asm volatile("cp.async.wait_group %0;" ::"n"(N) : "memory"); }
+
 inline int cdiv(int64_t a, int64_t b) { return (int)((a + b - 1) / b); }
+
+// SMs of the current device (persistent-kernel grids); 148 (B200) when the query fails
+inline int sm_count() {
+  int dev = 0, sms = 148;
+  cudaGetDevice(&dev);
+  cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+  return sms;
+}
+// stored size of the input along a conv-resolution extent v: half behind nearest-up2, twice behind the 2x2 pool
+__host__ __device__ inline int stored_res(const iea_conv_desc& d, int v) {
+  return d.in_mode == IEA_IN_UP2 ? v / 2 : (d.in_mode == IEA_IN_POOL2 ? v * 2 : v);
+}
+// tensor-memory columns to allocate for `need` accumulator columns: a power of two, at least 32
+inline uint32_t tmem_cols_for(uint32_t need) {
+  uint32_t cols = 32;
+  while (cols < need) cols <<= 1;
+  return cols;
+}
 
 }  // namespace iea

@@ -46,25 +46,7 @@ struct Params {
   uint32_t off_y, off_x, off_xt, off_tab, buf_bytes, off_w, off_stage, off_bar, stage_ld, tmem_cols;
 };
 
-__host__ __device__ constexpr uint32_t idesc_kk(int n) {
-  return (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(n >> 3) << 17) | ((uint32_t)(128 >> 4) << 24);
-}
-__host__ __device__ constexpr uint32_t idesc_mn(int n) {
-  return idesc_kk(n) | (1u << 15) | (1u << 16);
-}
 __device__ __forceinline__ uint64_t desc_mn(uint32_t addr) { return make_desc(addr, 128, PL); }
-__device__ __forceinline__ void cp16(uint32_t dst, const void* src) {
-  asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(dst), "l"(src) : "memory");
-}
-__device__ __forceinline__ void unpack8f(const uint4& q, float* f) { unpack8(q, f); }
-__device__ __forceinline__ void tmem_ld16_issue(uint32_t taddr, uint32_t* r) {
-  asm volatile(
-      "tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15}, [%16];"
-      : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]), "=r"(r[8]),
-        "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15])
-      : "r"(taddr));
-}
-__device__ __forceinline__ void tmem_ld_wait() { asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory"); }
 
 __global__ void __launch_bounds__(THREADS, 1) bwd1x1_kernel(const Params p) {
   extern __shared__ __align__(128) uint8_t smem[];
@@ -91,12 +73,9 @@ __global__ void __launch_bounds__(THREADS, 1) bwd1x1_kernel(const Params p) {
       mbar_init(d1_empty(b), 4);
     }
     mbar_init(d2_full, 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    fence_mbar_init();
   }
-  if (warp == 16) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)), "r"(p.tmem_cols));
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;");
-  }
+  if (warp == 16) tmem_alloc(smem_u32(tmem_slot), p.tmem_cols);
   // one-time shared-memory images: the resident dgrad weights and the ones plane behind xt (bias-gradient column of
   // MMA2).  Neither geff^T (A of MMA2, 128 rows) nor [xt | 1] (B, Cin + 16 columns) is padded: the descriptors simply
   // run on into whatever follows the real planes -- those operand rows / columns only produce accumulator rows >= Cout
@@ -132,14 +111,14 @@ __global__ void __launch_bounds__(THREADS, 1) bwd1x1_kernel(const Params p) {
         tc_fence_after();
         const uint32_t g0 = sbase + b * p.buf_bytes;
         if (p.want_x) {
-          const uint32_t w0 = sbase + p.off_w, id1 = idesc_kk(cin);
+          const uint32_t w0 = sbase + p.off_w, id1 = idesc(cin, false, false);
           for (int j = 0; j < cout / 16; ++j)
             tc_mma(tmem + db * cin, make_desc(g0 + 2 * j * PL, PL, 128), make_desc(w0 + 2 * j * (cin * 16), cin * 16, 128), id1,
                    j > 0 ? 1u : 0u);
           tc_commit(d1_full(db));
         }
         if (p.want_w) {
-          const uint32_t x0 = g0 + p.off_xt, id2 = idesc_mn(cin + 16);
+          const uint32_t x0 = g0 + p.off_xt, id2 = idesc(cin + 16, true, true);
 #pragma unroll
           for (int j = 0; j < BM / 16; ++j)
             tc_mma(tmem + 2 * cin, desc_mn(g0 + j * 256), desc_mn(x0 + j * 256), id2, (i > 0 || j > 0) ? 1u : 0u);
@@ -191,7 +170,7 @@ __global__ void __launch_bounds__(THREADS, 1) bwd1x1_kernel(const Params p) {
 #pragma unroll 2
         for (int k = 0; k < p.x_planes; ++k, src += x_gs, dst += xrs * 16) cp16(dst, src);
       }
-      asm volatile("cp.async.commit_group;" ::: "memory");
+      cp_async_commit();
       is_m0 += 2 * BM;
       is_b += 2;
       while (is_b >= nbuf) { is_b -= nbuf; ++is_u; }
@@ -232,9 +211,9 @@ __global__ void __launch_bounds__(THREADS, 1) bwd1x1_kernel(const Params p) {
       {  // the copies of this tile have landed; the younger requests stay in flight
         const int pend = PDg > 0 ? PDg - 1 : 0;
         const int younger = kmax - 1 - k < pend ? kmax - 1 - k : pend;
-        if (younger <= 0) asm volatile("cp.async.wait_group 0;" ::: "memory");
-        else if (younger == 1) asm volatile("cp.async.wait_group 1;" ::: "memory");
-        else asm volatile("cp.async.wait_group 2;" ::: "memory");
+        if (younger <= 0) cp_async_wait<0>();
+        else if (younger == 1) cp_async_wait<1>();
+        else cp_async_wait<2>();
       }
       // every copy of the group and the table are visible to the group
       if (pg == 0) asm volatile("bar.sync 1, 128;" ::: "memory");
@@ -244,8 +223,8 @@ __global__ void __launch_bounds__(THREADS, 1) bwd1x1_kernel(const Params p) {
 #pragma unroll 2
         for (int kk = 0; kk < p.g_planes; ++kk, q0 += grs * 16) {
           float gv[8], yv[8];
-          unpack8f(*reinterpret_cast<const uint4*>(q0), gv);
-          unpack8f(*reinterpret_cast<const uint4*>(q0 + p.off_y), yv);
+          unpack8(*reinterpret_cast<const uint4*>(q0), gv);
+          unpack8(*reinterpret_cast<const uint4*>(q0 + p.off_y), yv);
 #pragma unroll
           for (int j = 0; j < 8; ++j) gv[j] += fmaf(yv[j], e2[j], e1[j]);
           *reinterpret_cast<uint4*>(q0) = pack8(gv);
@@ -259,7 +238,7 @@ __global__ void __launch_bounds__(THREADS, 1) bwd1x1_kernel(const Params p) {
 #pragma unroll 2
           for (int kk = 0; kk < p.x_planes; ++kk, q0 += xrs * 16) {
             float xv[8];
-            unpack8f(*reinterpret_cast<const uint4*>(q0), xv);
+            unpack8(*reinterpret_cast<const uint4*>(q0), xv);
 #pragma unroll
             for (int j = 0; j < 8; ++j) xv[j] = fmaxf(fmaf(xv[j], sc[j], sh[j]), lo);
             *reinterpret_cast<uint4*>(q0 + to_xt) = pack8(xv);
@@ -355,7 +334,7 @@ __global__ void __launch_bounds__(THREADS, 1) bwd1x1_kernel(const Params p) {
         for (int q8 = 0; q8 < 2; ++q8) {  // 8 channels at a time
           const int c0 = c16 + q8 * 8;
           float xv[8], o[8], gm[8], ts[8], th[8];
-          unpack8f(xq[q8], xv);
+          unpack8(xq[q8], xv);
           if (d.in_scale) {  // 16-byte broadcast reads of the per-channel table
             const float4* t4 = reinterpret_cast<const float4*>(tab + c0);
             const float4* h4 = reinterpret_cast<const float4*>(tab + cin + c0);
@@ -379,7 +358,7 @@ __global__ void __launch_bounds__(THREADS, 1) bwd1x1_kernel(const Params p) {
           if (dxrow) {
             if (a.beta != 0.f) {
               float old[8];
-              unpack8f(oq[q8], old);
+              unpack8(oq[q8], old);
 #pragma unroll
               for (int j = 0; j < 8; ++j) o[j] = fmaf(a.beta, old[j], o[j]);
             }
@@ -397,8 +376,8 @@ __global__ void __launch_bounds__(THREADS, 1) bwd1x1_kernel(const Params p) {
         const uint8_t* xpl = buf + p.off_x + sc_c * PL;
         for (int r = r0; r < r0 + rows_q; ++r) {
           float gv[8], xr[8];
-          unpack8f(*reinterpret_cast<const uint4*>(stage + r * p.stage_ld + sc_c * 16), gv);
-          unpack8f(*reinterpret_cast<const uint4*>(xpl + r * 16), xr);
+          unpack8(*reinterpret_cast<const uint4*>(stage + r * p.stage_ld + sc_c * 16), gv);
+          unpack8(*reinterpret_cast<const uint4*>(xpl + r * 16), xr);
 #pragma unroll
           for (int j = 0; j < 8; ++j) { acc_h[j] += gv[j]; acc_s[j] = fmaf(gv[j], xr[j], acc_s[j]); }
         }
@@ -434,7 +413,7 @@ __global__ void __launch_bounds__(THREADS, 1) bwd1x1_kernel(const Params p) {
   }
   tc_fence_before();
   __syncthreads();
-  if (warp == 16) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem), "r"(p.tmem_cols));
+  if (warp == 16) tmem_free(tmem, p.tmem_cols);
 }
 
 // dscale / dshift [n][cin]: fixed-order sum of the partials of the CTAs that touched image n
@@ -498,9 +477,7 @@ static bool plan(const iea_conv_desc* d, const iea_bwd1x1_args* a, Params* p) {
   return true;
 }
 static int grid_of(const Params& p) {
-  int dev = 0, sms = 148;
-  cudaGetDevice(&dev);
-  cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+  const int sms = sm_count();
   return p.tiles < sms ? p.tiles : sms;
 }
 static void layout(Params* p, int grid) {

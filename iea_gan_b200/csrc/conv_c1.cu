@@ -16,21 +16,6 @@ using namespace iea;
 
 namespace c1 {
 
-__device__ __forceinline__ float2 ffma2(float2 a, float2 b, float2 c) {
-  float2 d;
-  asm("fma.rn.f32x2 %0, %1, %2, %3;" : "=l"(reinterpret_cast<unsigned long long&>(d))
-      : "l"(reinterpret_cast<unsigned long long&>(a)), "l"(reinterpret_cast<unsigned long long&>(b)),
-        "l"(reinterpret_cast<unsigned long long&>(c)));
-  return d;
-}
-__device__ __forceinline__ float2 bf2_to_f2(uint32_t w) {
-  return make_float2(__uint_as_float(w << 16), __uint_as_float(w & 0xFFFF0000u));
-}
-__device__ __forceinline__ uint32_t pack2(float a, float b) {
-  __nv_bfloat162 t = __floats2bfloat162_rn(a, b);
-  return *reinterpret_cast<uint32_t*>(&t);
-}
-
 struct Geo { int64_t n; int h, w; int64_t groups; };  // groups = n*h*(w/4) pixel quads
 
 // 3 x 6 window of the single-channel tensor around pixel quad (nn, hh, w0..w0+3); zero outside the image
@@ -198,9 +183,7 @@ __global__ void __launch_bounds__(256) c1_wgrad_kernel(const WgP p, const Geo g)
 
 inline bool al16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15) == 0; }
 inline int grid_for(int64_t groups, int cgn) {
-  int dev = 0, sms = 148;
-  cudaGetDevice(&dev);
-  cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+  const int sms = sm_count();
   const int64_t per_block = 256 / cgn;
   int64_t blocks = (groups + per_block - 1) / per_block;
   if (blocks > sms * 4) blocks = sms * 4;

@@ -20,8 +20,8 @@ __host__ __device__ inline Geo make_geo(const iea_conv_desc& d) {
   Geo g;
   g.M = d.n * (int64_t)d.h * d.w;
   g.K = d.cin * d.ksize * d.ksize;
-  g.hs = d.in_mode == IEA_IN_UP2 ? d.h / 2 : (d.in_mode == IEA_IN_POOL2 ? d.h * 2 : d.h);
-  g.ws = d.in_mode == IEA_IN_UP2 ? d.w / 2 : (d.in_mode == IEA_IN_POOL2 ? d.w * 2 : d.w);
+  g.hs = stored_res(d, d.h);
+  g.ws = stored_res(d, d.w);
   return g;
 }
 
@@ -394,17 +394,6 @@ extern "C" int iea_conv_wgrad(const iea_conv_desc* d, const void* g, int g_dtype
 // vectorised version for bf16 tensors with cin % 8 == 0: grid (pixel chunks, n), 256 threads =
 // (cin/8 sixteen-byte columns) x (pixel lanes); per-CTA partial (dscale, dshift) then a fixed-order reduce.
 namespace {
-__device__ __forceinline__ void unpack8v(const uint4& q, float* f) {
-  const uint32_t w[4] = {q.x, q.y, q.z, q.w};
-#pragma unroll
-  for (int i = 0; i < 4; ++i) { f[2 * i] = __uint_as_float(w[i] << 16); f[2 * i + 1] = __uint_as_float(w[i] & 0xFFFF0000u); }
-}
-__device__ __forceinline__ uint4 pack8v(const float* f) {
-  uint4 r; uint32_t* o = reinterpret_cast<uint32_t*>(&r);
-#pragma unroll
-  for (int i = 0; i < 4; ++i) { __nv_bfloat162 t = __floats2bfloat162_rn(f[2 * i], f[2 * i + 1]); o[i] = *reinterpret_cast<uint32_t*>(&t); }
-  return r;
-}
 __global__ void __launch_bounds__(256) conv_input_bwd_vec(const iea_conv_desc d, const Geo g, const bf16* __restrict__ da,
                                                           bf16* __restrict__ dx, int dx_ld, float beta, float* part,
                                                           int chunks, int px_per_chunk) {
@@ -431,7 +420,7 @@ __global__ void __launch_bounds__(256) conv_input_bwd_vec(const iea_conv_desc d,
     for (int p = p0 + pl; p < p1; p += lanes) {
       const int xh = p / g.ws, xw = p - xh * g.ws;
       float xv[8], gs[8];
-      unpack8v(__ldg(reinterpret_cast<const uint4*>(xb + (n * npx + p) * d.x_ld + c0)), xv);
+      unpack8(__ldg(reinterpret_cast<const uint4*>(xb + (n * npx + p) * d.x_ld + c0)), xv);
       if (d.in_mode == IEA_IN_UP2) {
 #pragma unroll
         for (int j = 0; j < 8; ++j) gs[j] = 0.f;
@@ -440,16 +429,16 @@ __global__ void __launch_bounds__(256) conv_input_bwd_vec(const iea_conv_desc d,
 #pragma unroll
           for (int b = 0; b < 2; ++b) {
             float t[8];
-            unpack8v(__ldg(reinterpret_cast<const uint4*>(da + ((n * d.h + 2 * xh + a) * (int64_t)d.w + 2 * xw + b) * d.cin + c0)), t);
+            unpack8(__ldg(reinterpret_cast<const uint4*>(da + ((n * d.h + 2 * xh + a) * (int64_t)d.w + 2 * xw + b) * d.cin + c0)), t);
 #pragma unroll
             for (int j = 0; j < 8; ++j) gs[j] += t[j];
           }
       } else if (d.in_mode == IEA_IN_POOL2) {
-        unpack8v(__ldg(reinterpret_cast<const uint4*>(da + ((n * d.h + (xh >> 1)) * (int64_t)d.w + (xw >> 1)) * d.cin + c0)), gs);
+        unpack8(__ldg(reinterpret_cast<const uint4*>(da + ((n * d.h + (xh >> 1)) * (int64_t)d.w + (xw >> 1)) * d.cin + c0)), gs);
 #pragma unroll
         for (int j = 0; j < 8; ++j) gs[j] *= 0.25f;
       } else {
-        unpack8v(__ldg(reinterpret_cast<const uint4*>(da + (n * npx + p) * d.cin + c0)), gs);
+        unpack8(__ldg(reinterpret_cast<const uint4*>(da + (n * npx + p) * d.cin + c0)), gs);
       }
       float o[8];
 #pragma unroll
@@ -464,11 +453,11 @@ __global__ void __launch_bounds__(256) conv_input_bwd_vec(const iea_conv_desc d,
         bf16* q = dx + (n * npx + p) * dx_ld + c0;
         if (beta != 0.f) {
           float old[8];
-          unpack8v(*reinterpret_cast<const uint4*>(q), old);
+          unpack8(*reinterpret_cast<const uint4*>(q), old);
 #pragma unroll
           for (int j = 0; j < 8; ++j) o[j] = fmaf(beta, old[j], o[j]);
         }
-        *reinterpret_cast<uint4*>(q) = pack8v(o);
+        *reinterpret_cast<uint4*>(q) = pack8(o);
       }
     }
   if (part) {
@@ -639,8 +628,8 @@ __global__ void __launch_bounds__(256) conv_out_bwd_vec(const bf16* dy, int dy_l
       if (!ok[u]) continue;
       const int64_t m = m0 + u * stride;
       float v[8], yv[8];
-      unpack8v(qd[u], v);
-      if (need_y) unpack8v(qy[u], yv);
+      unpack8(qd[u], v);
+      if (need_y) unpack8(qy[u], yv);
       if (act == IEA_ACT_TANH) {
 #pragma unroll
         for (int j = 0; j < 8; ++j) v[j] *= (1.f - yv[j] * yv[j]);
@@ -655,7 +644,10 @@ __global__ void __launch_bounds__(256) conv_out_bwd_vec(const bf16* dy, int dy_l
 #pragma unroll
         for (int j = 0; j < 8; ++j) v[j] += fmaf(2.f * yv[j], t[j], s[j]);
       }
-      *reinterpret_cast<uint4*>(gout + m * c + cgi * 8) = pack8v(v);
+      uint32_t o[4];  // (pack2 in a loop, not pack8: with pack8 the compiler unswitches the row loop into three copies)
+#pragma unroll
+      for (int j = 0; j < 4; ++j) o[j] = pack2(v[2 * j], v[2 * j + 1]);
+      *reinterpret_cast<uint4*>(gout + m * c + cgi * 8) = make_uint4(o[0], o[1], o[2], o[3]);
     }
   }
 }
@@ -678,14 +670,14 @@ __global__ void __launch_bounds__(256) colsum_part_vec(const bf16* g, int g_ld, 
 #pragma unroll
       for (int u = 0; u < 4; ++u) {
         float f[8];
-        unpack8v(q[u], f);
+        unpack8(q[u], f);
 #pragma unroll
         for (int j = 0; j < 8; ++j) a[j] += f[j];
       }
     }
     for (; m < r1; m += lanes) {
       float f[8];
-      unpack8v(ld_nc16(g + m * g_ld + cgi * 8), f);
+      unpack8(ld_nc16(g + m * g_ld + cgi * 8), f);
 #pragma unroll
       for (int j = 0; j < 8; ++j) a[j] += f[j];
     }
@@ -728,7 +720,7 @@ __global__ void residual_bwd_vec(const bf16* g, int g_ld, int64_t n, int h, int 
     for (int j = 0; j < 8; ++j) v[j] = 0.f;
     if (c0 < res_c) {
       if (res_mode == IEA_IN_DIRECT) {
-        unpack8v(*reinterpret_cast<const uint4*>(g + p * g_ld + c0), v);
+        unpack8(*reinterpret_cast<const uint4*>(g + p * g_ld + c0), v);
       } else {
         int xw, xh; int64_t nn;
         if (small) {
@@ -746,12 +738,12 @@ __global__ void residual_bwd_vec(const bf16* g, int g_ld, int64_t n, int h, int 
 #pragma unroll
             for (int b = 0; b < 2; ++b) {
               float f[8];
-              unpack8v(*reinterpret_cast<const uint4*>(g + ((nn * h + 2 * xh + a) * (int64_t)w + 2 * xw + b) * g_ld + c0), f);
+              unpack8(*reinterpret_cast<const uint4*>(g + ((nn * h + 2 * xh + a) * (int64_t)w + 2 * xw + b) * g_ld + c0), f);
 #pragma unroll
               for (int j = 0; j < 8; ++j) v[j] += f[j];
             }
         } else {
-          unpack8v(*reinterpret_cast<const uint4*>(g + ((nn * h + (xh >> 1)) * (int64_t)w + (xw >> 1)) * g_ld + c0), v);
+          unpack8(*reinterpret_cast<const uint4*>(g + ((nn * h + (xh >> 1)) * (int64_t)w + (xw >> 1)) * g_ld + c0), v);
 #pragma unroll
           for (int j = 0; j < 8; ++j) v[j] *= 0.25f;
         }
@@ -760,11 +752,11 @@ __global__ void residual_bwd_vec(const bf16* g, int g_ld, int64_t n, int h, int 
     bf16* q = dres + p * dres_ld + c0;
     if (beta != 0.f) {
       float old[8];
-      unpack8v(*reinterpret_cast<const uint4*>(q), old);
+      unpack8(*reinterpret_cast<const uint4*>(q), old);
 #pragma unroll
       for (int j = 0; j < 8; ++j) v[j] = fmaf(beta, old[j], v[j]);
     }
-    *reinterpret_cast<uint4*>(q) = pack8v(v);
+    *reinterpret_cast<uint4*>(q) = pack8(v);
   }
 }
 inline bool al16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15) == 0; }

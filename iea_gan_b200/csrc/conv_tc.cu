@@ -205,13 +205,9 @@ __global__ void __launch_bounds__(THREADS, 1) conv_tc_kernel(const Params p) {
     // mbarrier serialise and wake the parked MMA thread 128 times per step
     for (int s = 0; s < p.stages; ++s) { mbar_init(full_bar(s), NPT / 32 + 1); mbar_init(empty_bar(s), 1); }
     for (int b = 0; b < 2; ++b) { mbar_init(tfull_bar(b), 1); mbar_init(tempty_bar(b), 4); }
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    fence_mbar_init();
   }
-  if (warp == 0) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)),
-                 "r"(p.tmem_cols));
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;");
-  }
+  if (warp == 0) tmem_alloc(smem_u32(tmem_slot), p.tmem_cols);
   tc_fence_before();
   __syncthreads();
   tc_fence_after();
@@ -223,7 +219,7 @@ __global__ void __launch_bounds__(THREADS, 1) conv_tc_kernel(const Params p) {
   if (warp == 0) {
     // ===================== MMA issuer =====================
     if (lane == 0) {
-      const uint32_t idesc = (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(p.BN >> 3) << 17) | ((uint32_t)(BM >> 4) << 24);
+      const uint32_t id = idesc(p.BN, false, false);
       uint32_t g = 0, tcount = 0;
       for (int tile = blockIdx.x; tile < num_tiles; tile += gridDim.x, ++tcount) {
         const uint32_t ab = tcount & 1, aph = (tcount >> 1) & 1;
@@ -239,7 +235,7 @@ __global__ void __launch_bounds__(THREADS, 1) conv_tc_kernel(const Params p) {
           for (int j = 0; j < CPR / 2; ++j) {
             const uint64_t da = make_desc(a0 + 2 * j * p.lbo_a, p.lbo_a, 128);
             const uint64_t db = make_desc(b0 + 2 * j * p.lbo_b, p.lbo_b, 128);
-            tc_mma(tacc, da, db, idesc, (it > 0 || j > 0) ? 1u : 0u);
+            tc_mma(tacc, da, db, id, (it > 0 || j > 0) ? 1u : 0u);
           }
           tc_commit(empty_bar(s));
         }
@@ -424,7 +420,7 @@ __global__ void __launch_bounds__(THREADS, 1) conv_tc_kernel(const Params p) {
   __syncthreads();
   if (warp == 0) {
     tc_fence_after();
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(p.tmem_cols));
+    tmem_free(tmem_base, p.tmem_cols);
   }
 }
 
@@ -462,13 +458,9 @@ __global__ void __launch_bounds__(LR_THREADS, 1) conv_lr_kernel(const Params p) 
       mbar_init(pfull_bar(b), LR_NPT / 32); mbar_init(pempty_bar(b), 1);  // one arrival per producer warp
       mbar_init(tfull_bar(b), 1); mbar_init(tempty_bar(b), 4);
     }
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    fence_mbar_init();
   }
-  if (warp == 0) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)),
-                 "r"(p.tmem_cols));
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;");
-  }
+  if (warp == 0) tmem_alloc(smem_u32(tmem_slot), p.tmem_cols);
   tc_fence_before();
   __syncthreads();
   tc_fence_after();
@@ -478,7 +470,7 @@ __global__ void __launch_bounds__(LR_THREADS, 1) conv_lr_kernel(const Params p) 
   if (warp == 0) {
     // ===================== MMA issuer =====================
     if (lane == 0) {
-      const uint32_t idesc = (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(p.BN >> 3) << 17) | ((uint32_t)(BM >> 4) << 24);
+      const uint32_t id = idesc(p.BN, false, false);
       const uint64_t da0 = make_desc(sbase, p.plane, 160);
       const uint64_t db0 = make_desc(sbase + p.ring_off, p.lbo_b, 128);
       const uint32_t plane16 = p.plane >> 4, lbo16 = p.lbo_b >> 4, stage16 = p.b_bytes >> 4, patch16 = p.patch_bytes >> 4;
@@ -497,7 +489,7 @@ __global__ void __launch_bounds__(LR_THREADS, 1) conv_lr_kernel(const Params p) 
             const uint32_t a16 = a_tap + kb * LR_CPR * plane16, b16 = s * stage16;
 #pragma unroll
             for (int j = 0; j < LR_CPR / 2; ++j)
-              tc_mma(tacc, da0 + (a16 + 2 * j * plane16), db0 + (b16 + 2 * j * lbo16), idesc,
+              tc_mma(tacc, da0 + (a16 + 2 * j * plane16), db0 + (b16 + 2 * j * lbo16), id,
                      (tap > 0 || kb > 0 || j > 0) ? 1u : 0u);
             tc_commit(wempty_bar(s));
             if (++s == (uint32_t)p.stages) { s = 0; ph ^= 1; }
@@ -625,7 +617,7 @@ __global__ void __launch_bounds__(LR_THREADS, 1) conv_lr_kernel(const Params p) 
   __syncthreads();
   if (warp == 0) {
     tc_fence_after();
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(p.tmem_cols));
+    tmem_free(tmem_base, p.tmem_cols);
   }
 }
 
@@ -669,8 +661,8 @@ int iea_conv_fprop_tc(const iea_conv_desc* d, cudaStream_t s) {
   p.d = *d;
   p.wtc = (const bf16*)d->wpack_tc;
   p.M = d->n * (int64_t)d->h * d->w;
-  p.hs = d->in_mode == IEA_IN_UP2 ? d->h / 2 : (d->in_mode == IEA_IN_POOL2 ? d->h * 2 : d->h);
-  p.ws = d->in_mode == IEA_IN_UP2 ? d->w / 2 : (d->in_mode == IEA_IN_POOL2 ? d->w * 2 : d->w);
+  p.hs = stored_res(*d, d->h);
+  p.ws = stored_res(*d, d->w);
   p.KB = d->cin < 64 ? d->cin : 64;
   p.nkb = d->cin / p.KB;
   p.taps = d->ksize * d->ksize;
@@ -699,12 +691,9 @@ int iea_conv_fprop_tc(const iea_conv_desc* d, cudaStream_t s) {
   p.bar_off = p.tab_off + tab_bytes;
   p.tfull_off = 8u * 2 * stages;
   const uint32_t smem = p.bar_off + 256;
-  uint32_t cols = 32;
-  while (cols < (uint32_t)(2 * p.BN)) cols <<= 1;
+  const uint32_t cols = tmem_cols_for(2 * p.BN);
   p.tmem_cols = cols;
-  int dev = 0, sms = 148;
-  cudaGetDevice(&dev);
-  cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+  const int sms = sm_count();
   const int tiles = p.n_tiles_m * p.n_tiles_n;
   const int occ = (smem <= 100 * 1024 && cols <= 256) ? 2 : 1;
   int grid = tiles < sms * occ ? tiles : sms * occ;
@@ -776,20 +765,16 @@ int iea_conv_fprop_lowres(const iea_conv_desc* d, cudaStream_t s) {
   p.d = *d;
   p.wtc = (const bf16*)d->wpack_tc;
   p.M = d->n * (int64_t)d->h * d->w;
-  p.hs = d->in_mode == IEA_IN_UP2 ? d->h / 2 : d->h;
-  p.ws = d->in_mode == IEA_IN_UP2 ? d->w / 2 : d->w;
+  p.hs = stored_res(*d, d->h);
+  p.ws = stored_res(*d, d->w);
   p.KB = 64;
   p.nkb = d->cin / 64;
   p.taps = 9;
   p.n_tiles_n = 1;
   p.n_tiles_m = (int)((p.M + tc::BM - 1) / tc::BM);
   const uint32_t smem = p.bar_off + 256;
-  uint32_t cols = 32;
-  while (cols < (uint32_t)(2 * p.BN)) cols <<= 1;
-  p.tmem_cols = cols;
-  int dev = 0, sms = 148;
-  cudaGetDevice(&dev);
-  cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+  p.tmem_cols = tmem_cols_for(2 * p.BN);
+  const int sms = sm_count();
   const int grid = p.n_tiles_m < sms ? p.n_tiles_m : sms;
   IEA_CUDA(cudaFuncSetAttribute(tc::conv_lr_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   tc::conv_lr_kernel<<<grid, tc::LR_THREADS, smem, s>>>(p);

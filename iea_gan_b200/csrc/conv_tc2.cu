@@ -16,7 +16,6 @@
 // Layers whose weights do not fit (>= 128-channel 3x3, 512-channel 1x1) use the streaming kernel.
 #include "tc_common.cuh"
 #include <type_traits>
-#include <stdlib.h>
 using namespace iea;
 
 namespace tc2 {
@@ -26,47 +25,12 @@ constexpr int BM = 128;
 constexpr int THREADS = 288;
 constexpr int PW = 10, PH = 18;  // 3x3 halo patch of a 16x8 tile
 
-// n / d for 0 <= n < 2^31 via one multiply-high (d fixed per launch)
-struct FastDiv { uint32_t mul, shr, d; };
-inline FastDiv make_fastdiv(uint32_t d) {
-  FastDiv f; f.d = d;
-  if (d == 1) { f.mul = 0; f.shr = 0; return f; }
-  uint32_t s = 0;
-  while ((1u << s) < d) ++s;
-  f.shr = s;
-  f.mul = (uint32_t)(((1ull << (32 + s)) + d - 1) / d - (1ull << 32));  // round-up magic (Granlund-Montgomery)
-  return f;
-}
-__device__ __forceinline__ uint32_t fdiv(uint32_t n, const FastDiv& f) {
-  if (f.d == 1) return n;
-  const uint32_t t = __umulhi(n, f.mul);
-  return (t + ((n - t) >> 1)) >> (f.shr - 1);
-}
-
-#ifdef IEA_TC2_TRACE
-// pipeline trace of CTA 0 (profiling builds only): clock64 stamps per role and item
-__device__ long long g_trace[8][512];
-#define TRACE(slot, idx) do { if (blockIdx.x == 0 && (idx) < 512) g_trace[slot][idx] = clock64(); } while (0)
-#else
-#define TRACE(slot, idx) do { } while (0)
-#endif
-
-// ablation switches of the profiling builds (-DIEA_THIN_DBG, IEA_TC2_DBG bits as in tools/ablate.py);
-// compiled out of the product kernel
-#ifdef IEA_THIN_DBG
-#define DBG(bit) (p.dbg & (bit))
-#define DBG_ANY (p.dbg != 0)
-#else
-#define DBG(bit) 0
-#define DBG_ANY 0
-#endif
-
 struct Params {
   FastDiv fd_tw, fd_th, fd_w, fd_h, fd_hw, fd_tpe;  // fd_tpe: tiles per event (lean-epilogue statistics slots)
   iea_conv_desc d;
   const bf16* wtc;
   int64_t M;
-  int n_tiles, hw, hs, ws, KB, nkb, BN, taps, tiles_w, tiles_h, npix, stages, uniform_n, depth, dbg, occ;
+  int n_tiles, hw, hs, ws, KB, nkb, BN, taps, tiles_w, tiles_h, npix, stages, uniform_n, depth;
   uint32_t plane, stage_bytes, w_bytes, stage_off, staging_off, staging_ld, stat_off, bar_off, tmem_cols;
 };
 
@@ -108,22 +72,6 @@ __device__ __forceinline__ Origin origin_of(const TilePos& c, int tile) {
   else { o.m0 = (int64_t)tile * BM; o.n = 0; o.h0 = 0; o.w0 = 0; }
   return o;
 }
-
-// packed fp32 pairs (Blackwell FFMA2 / FADD2): half the issue slots of scalar fp32 in the epilogue
-__device__ __forceinline__ float2 ffma2(float2 a, float2 b, float2 c) {
-  float2 r;
-  asm("fma.rn.f32x2 %0, %1, %2, %3;" : "=l"(reinterpret_cast<unsigned long long&>(r))
-      : "l"(reinterpret_cast<unsigned long long&>(a)), "l"(reinterpret_cast<unsigned long long&>(b)),
-        "l"(reinterpret_cast<unsigned long long&>(c)));
-  return r;
-}
-__device__ __forceinline__ float2 fadd2(float2 a, float2 b) {
-  float2 r;
-  asm("add.rn.f32x2 %0, %1, %2;" : "=l"(reinterpret_cast<unsigned long long&>(r))
-      : "l"(reinterpret_cast<unsigned long long&>(a)), "l"(reinterpret_cast<unsigned long long&>(b)));
-  return r;
-}
-__device__ __forceinline__ float2 bf2_to_f2(uint32_t w) { return make_float2(__uint_as_float(w << 16), __uint_as_float(w & 0xFFFF0000u)); }
 
 __device__ __forceinline__ uint4 transform(const uint4& raw, const float* sc, const float* sh, bool affine, bool relu) {
   float f[8];
@@ -167,13 +115,9 @@ __global__ void __launch_bounds__(THREADS, OCC) conv_tc2_kernel(const Params p) 
     for (int s = 0; s < p.stages; ++s) { mbar_init(full_bar(s), 4); mbar_init(empty_bar(s), 1); }
     for (int b = 0; b < 2; ++b) { mbar_init(tfull_bar(b), 1); mbar_init(tempty_bar(b), 4); }
     mbar_init(w_bar, 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    fence_mbar_init();
   }
-  if (warp == 0) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)),
-                 "r"(p.tmem_cols));
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;");
-  }
+  if (warp == 0) tmem_alloc(smem_u32(tmem_slot), p.tmem_cols);
   tc_fence_before();
   __syncthreads();
   tc_fence_after();
@@ -193,7 +137,7 @@ __global__ void __launch_bounds__(THREADS, OCC) conv_tc2_kernel(const Params p) 
         bulk_g2s(sbase + off, (const uint8_t*)p.wtc + off, nb, w_bar);
       }
       mbar_wait(w_bar, 0);
-      const uint32_t idesc = (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(p.BN >> 3) << 17) | ((uint32_t)(BM >> 4) << 24);
+      const uint32_t id = idesc(p.BN, false, false);
       const uint32_t lbo_b = p.BN * 16;
       const uint32_t sbo_a = IS3 ? PW * 16 : 128;
       // descriptors differ only in their 16-byte-unit start address: build the two bases once and add offsets
@@ -209,7 +153,6 @@ __global__ void __launch_bounds__(THREADS, OCC) conv_tc2_kernel(const Params p) 
         for (int kb = 0; kb < p.nkb; ++kb) {
           mbar_wait(full_bar(s), ph);
           tc_fence_after();
-          TRACE(3, tcount);
           const uint32_t a16 = s * stage16;
 #pragma unroll
           for (int tap = 0; tap < TAPS; ++tap) {
@@ -219,14 +162,13 @@ __global__ void __launch_bounds__(THREADS, OCC) conv_tc2_kernel(const Params p) 
             for (int j = 0; j < CPR / 2; ++j) {
               const uint64_t da = da_base + (a_tap + 2 * j * plane16);
               const uint64_t db = db_base + (b_tap + 2 * j * lbo16);
-              if (!DBG(2)) tc_mma(tacc, da, db, idesc, (kb > 0 || tap > 0 || j > 0) ? 1u : 0u);
+              tc_mma(tacc, da, db, id, (kb > 0 || tap > 0 || j > 0) ? 1u : 0u);
             }
           }
           tc_commit(empty_bar(s));
           if (++s == (uint32_t)p.stages) { s = 0; ph ^= 1; }
         }
         tc_commit(tfull_bar(ab));
-        TRACE(4, tcount);
       }
     }
   } else if (warp <= 4) {
@@ -302,12 +244,9 @@ __global__ void __launch_bounds__(THREADS, OCC) conv_tc2_kernel(const Params p) 
         if (IS3) base = ((int64_t)(c.t.n * p.hs + ((c.t.th * 16) >> sh_)) * p.ws + ((c.t.tw * 8) >> sh_)) * d.x_ld + ci;
         else base = (int64_t)(tile0 + c.tl) * BM * d.x_ld + ci;
         const bf16* bp = xb + base;
-        if (!DBG(16)) {
 #pragma unroll
-          for (int i = 0; i < NL; ++i)
-            if (i < NL - 1 || last_ok)
-              asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(a1 + i * GP * 16), "l"(bp + dlt[i]) : "memory");
-        }
+        for (int i = 0; i < NL; ++i)
+          if (i < NL - 1 || last_ok) cp16(a1 + i * GP * 16, bp + dlt[i]);
         return;
       }
       const Origin o = origin_of<IS3>(c.t, tile0 + c.tl);
@@ -329,8 +268,8 @@ __global__ void __launch_bounds__(THREADS, OCC) conv_tc2_kernel(const Params p) 
           const float v = cc == 0 ? ld_act(d.x, d.x_dtype, pix * d.x_ld) : 0.f;
           const uint32_t lo = (uint32_t)__bfloat16_as_ushort(__float2bfloat16_rn(v));
           asm volatile("st.shared.v4.b32 [%0], {%1,%2,%2,%2};" ::"r"(a1 + i * GP * 16), "r"(lo), "r"(0) : "memory");
-        } else if (in && !DBG(16)) {
-          asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(a1 + i * GP * 16), "l"(xb + pix * d.x_ld + ci) : "memory");
+        } else if (in) {
+          cp16(a1 + i * GP * 16, xb + pix * d.x_ld + ci);
         } else {
           asm volatile("st.shared.v4.b32 [%0], {%1,%1,%1,%1};" ::"r"(a1 + i * GP * 16), "r"(0) : "memory");
         }
@@ -343,7 +282,7 @@ __global__ void __launch_bounds__(THREADS, OCC) conv_tc2_kernel(const Params p) 
     int issued = 0;
     for (int k = 0; k < D - 1; ++k) {
       if (issued < n_items) { issue(ci_); cur_next(ci_); ++issued; }
-      asm volatile("cp.async.commit_group;" ::: "memory");
+      cp_async_commit();
     }
     // fused prologue constants as packed bf16x2: relu(x*scale+shift) is ONE fma.rn.relu.bf16x2 per channel
     // pair (single rounding of the fused result; scale/shift carry bf16 precision like the weights do)
@@ -352,15 +291,14 @@ __global__ void __launch_bounds__(THREADS, OCC) conv_tc2_kernel(const Params p) 
     int ss_n = -1, ss_ci = -1;
     for (int it = 0; it < n_items; ++it) {
       if (issued < n_items) { issue(ci_); cur_next(ci_); ++issued; }
-      asm volatile("cp.async.commit_group;" ::: "memory");
+      cp_async_commit();
       switch (D) {  // wait until item `it` (this thread's part) has landed
-        case 2: asm volatile("cp.async.wait_group 1;" ::: "memory"); break;
-        case 3: asm volatile("cp.async.wait_group 2;" ::: "memory"); break;
-        case 4: asm volatile("cp.async.wait_group 3;" ::: "memory"); break;
-        case 6: asm volatile("cp.async.wait_group 5;" ::: "memory"); break;
-        default: asm volatile("cp.async.wait_group 0;" ::: "memory"); break;
+        case 2: cp_async_wait<1>(); break;
+        case 3: cp_async_wait<2>(); break;
+        case 4: cp_async_wait<3>(); break;
+        case 6: cp_async_wait<5>(); break;
+        default: cp_async_wait<0>(); break;
       }
-      if (pt == 0) TRACE(0, it);
       const Cur& c = ct_;
       const int ci = c.kb * p.KB + cc * 8;
       uint8_t* a1 = smem + (a_thr - sbase) + c.s * p.stage_bytes;
@@ -411,7 +349,7 @@ __global__ void __launch_bounds__(THREADS, OCC) conv_tc2_kernel(const Params p) 
           const bool in = coords_slow(o, pp, nn, ih, iw);
           *reinterpret_cast<uint4*>(a1 + i * GP * 16) = in ? load_chunk(d, p.hs, p.ws, nn, ih, iw, ci) : make_uint4(0, 0, 0, 0);
         }
-      } else if ((affine || relu) && !DBG(1)) {  // in-place fused prologue on the chunks this thread copied
+      } else if (affine || relu) {  // in-place fused prologue on the chunks this thread copied
         const int nn = c.t.n;  // (affine on a 1x1 layer implies uniform_n, so the cursor's image index is exact)
         if (affine && (nn != ss_n || ci != ss_ci)) {
           float sc[8], sh[8];
@@ -455,14 +393,12 @@ __global__ void __launch_bounds__(THREADS, OCC) conv_tc2_kernel(const Params p) 
           *q = v;
         }
       }
-      if (pt == 0) TRACE(1, it);
       fence_async_smem();
       __syncwarp();
       if (lane == 0) mbar_arrive(full_bar(c.s));
-      if (pt == 0) TRACE(2, it);
       cur_next(ct_);
     }
-    asm volatile("cp.async.wait_group 0;" ::: "memory");
+    cp_async_wait<0>();
   } else {
     // ===================== epilogue =====================
     const int q = warp & 3, et = q * 32 + lane;  // TMEM lane == tile row
@@ -541,10 +477,8 @@ __global__ void __launch_bounds__(THREADS, OCC) conv_tc2_kernel(const Params p) 
           if (ev_pos == tpe) { flush(ev); ++ev; ev_pos = 0; }
           ++ev_pos;
         }
-        if (et == 0) TRACE(5, tcount);
         mbar_wait(tfull_bar(ab), aph);
         tc_fence_after();
-        if (et == 0) TRACE(6, tcount);
 #pragma unroll
         for (int cb = 0; cb < LEANB; ++cb) {
           float2 v[8];
@@ -604,8 +538,8 @@ __global__ void __launch_bounds__(THREADS, OCC) conv_tc2_kernel(const Params p) 
           uint32_t o[8];
 #pragma unroll
           for (int j = 0; j < 8; ++j) o[j] = pack2(v[j].x, v[j].y);
-          if (!DBG(4)) { yp[0] = make_uint4(o[0], o[1], o[2], o[3]); yp[1] = make_uint4(o[4], o[5], o[6], o[7]); }
-          if (has_stats && !DBG(8)) {
+          yp[0] = make_uint4(o[0], o[1], o[2], o[3]); yp[1] = make_uint4(o[4], o[5], o[6], o[7]);
+          if (has_stats) {
 #pragma unroll
             for (int j = 0; j < 8; ++j) { s1[cb * 8 + j] = fadd2(s1[cb * 8 + j], v[j]); s2[cb * 8 + j] = ffma2(v[j], v[j], s2[cb * 8 + j]); }
           }
@@ -614,7 +548,6 @@ __global__ void __launch_bounds__(THREADS, OCC) conv_tc2_kernel(const Params p) 
         tc_fence_before();
         __syncwarp();
         if (lane == 0) mbar_arrive(tempty_bar(ab));
-        if (et == 0) TRACE(7, tcount);
       }
       if (has_stats && my_tiles > 0) flush(ev);
     } else {
@@ -629,7 +562,7 @@ __global__ void __launch_bounds__(THREADS, OCC) conv_tc2_kernel(const Params p) 
     // residual and statistics switches), packed fp32x2 math, copy-out with per-thread constant strides, and
     // the batch-norm partial sums taken from the 16-byte chunks while they are copied out (no second pass).
     const bool fast = d.acc_c0 < 0 && d.act == IEA_ACT_NONE && d.cout >= 16 && cg_pow2 && cg <= 32 &&
-                      (!d.res || d.res_mode != IEA_IN_POOL2) && !DBG_ANY;
+                      (!d.res || d.res_mode != IEA_IN_POOL2);
     auto fast_loop = [&](auto res_c_, auto stats_c_) {
       constexpr bool RES = decltype(res_c_)::value, STATS = decltype(stats_c_)::value;
       const int g8 = et & (cg - 1), r0 = et >> cg_sh, step = 128 >> cg_sh;  // copy-out: rows r0, r0+step, ... of chunk g8
@@ -665,12 +598,8 @@ __global__ void __launch_bounds__(THREADS, OCC) conv_tc2_kernel(const Params p) 
         for (int cb = 0; cb < ncb; ++cb) {
           const int c0 = cb * 16;
           uint32_t raw[16];
-          asm volatile(
-              "tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15}, [%16];"
-              : "=r"(raw[0]), "=r"(raw[1]), "=r"(raw[2]), "=r"(raw[3]), "=r"(raw[4]), "=r"(raw[5]), "=r"(raw[6]), "=r"(raw[7]),
-                "=r"(raw[8]), "=r"(raw[9]), "=r"(raw[10]), "=r"(raw[11]), "=r"(raw[12]), "=r"(raw[13]), "=r"(raw[14]), "=r"(raw[15])
-              : "r"(tmem_base + ((uint32_t)(q * 32) << 16) + ab * p.BN + c0));
-          asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+          tmem_ld16_issue(tmem_base + ((uint32_t)(q * 32) << 16) + ab * p.BN + c0, raw);
+          tmem_ld_wait();
           float2 v[8];
 #pragma unroll
           for (int j4 = 0; j4 < 4; ++j4) {
@@ -938,7 +867,7 @@ __global__ void __launch_bounds__(THREADS, OCC) conv_tc2_kernel(const Params p) 
   __syncthreads();
   if (warp == 0) {
     tc_fence_after();
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(p.tmem_cols));
+    tmem_free(tmem_base, p.tmem_cols);
   }
 }
 
@@ -976,16 +905,16 @@ int iea_conv_tc2_stats_slots(const iea_conv_desc* d) {
   return tc2_tiles_per_event(d);
 }
 
-// launch geometry shared by the launcher and the statistics-slot query
-static int tc2_prepare(const iea_conv_desc* d, tc2::Params& p, int& grid, uint32_t& smem_out, int& cpr_out, bool& is3_out) {
+// launch geometry shared by the launcher and the statistics-slot query; occ_out: CTAs per SM it is sized for
+static int tc2_prepare(const iea_conv_desc* d, tc2::Params& p, int& grid, uint32_t& smem_out, int& cpr_out, bool& is3_out,
+                       int& occ_out) {
   p.d = *d;
   p.wtc = (const bf16*)d->wpack_tc;
-  { const char* e_ = getenv("IEA_TC2_DBG"); p.dbg = e_ ? atoi(e_) : 0; }  // profiling ablations only
   p.M = d->n * (int64_t)d->h * d->w;
   p.hw = d->h * d->w;
-  p.fd_w = tc2::make_fastdiv(d->w); p.fd_h = tc2::make_fastdiv(d->h); p.fd_hw = tc2::make_fastdiv(p.hw);
-  p.hs = d->in_mode == IEA_IN_UP2 ? d->h / 2 : (d->in_mode == IEA_IN_POOL2 ? d->h * 2 : d->h);
-  p.ws = d->in_mode == IEA_IN_UP2 ? d->w / 2 : (d->in_mode == IEA_IN_POOL2 ? d->w * 2 : d->w);
+  p.fd_w = tc::make_fastdiv(d->w); p.fd_h = tc::make_fastdiv(d->h); p.fd_hw = tc::make_fastdiv(p.hw);
+  p.hs = stored_res(*d, d->h);
+  p.ws = stored_res(*d, d->w);
   const int cin_eff = d->cin < 16 ? 16 : d->cin;  // 1-channel stem: K padded to one 16-wide MMA step
   p.KB = cin_eff < 64 ? cin_eff : 64;
   p.nkb = cin_eff / p.KB;
@@ -997,7 +926,7 @@ static int tc2_prepare(const iea_conv_desc* d, tc2::Params& p, int& grid, uint32
   // 1x1: a "tile row" is one image when images are whole tiles; otherwise the column counter never wraps
   p.tiles_w = is3 ? d->w / 8 : (p.uniform_n ? p.hw / 128 : p.n_tiles + 1);
   p.tiles_h = is3 ? d->h / 16 : 1;
-  p.fd_tw = tc2::make_fastdiv(p.tiles_w); p.fd_th = tc2::make_fastdiv(p.tiles_h);
+  p.fd_tw = tc::make_fastdiv(p.tiles_w); p.fd_th = tc::make_fastdiv(p.tiles_h);
   p.npix = is3 ? tc2::PH * tc2::PW : 128;
   const int cpr = p.KB / 8;
   // planes (8 channels each) are skewed by 128 / CPR bytes: the CPR chunks of a pixel are copied / transformed by
@@ -1026,29 +955,23 @@ static int tc2_prepare(const iea_conv_desc* d, tc2::Params& p, int& grid, uint32
   p.stat_off = p.staging_off + staging_bytes;
   p.bar_off = p.stat_off + stat_bytes;
   const uint32_t smem = p.bar_off + 256 + 2 * p.BN * 4;
-  uint32_t cols = 32;
-  while (cols < (uint32_t)(2 * p.BN)) cols <<= 1;
+  const uint32_t cols = tmem_cols_for(2 * p.BN);
   p.tmem_cols = cols;
-  int dev = 0, sms = 148;
-  cudaGetDevice(&dev);
-  cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-  int occ = (cpr == 2 && smem <= 72 * 1024 && cols <= 128) ? 3 : ((cpr <= 4 && smem <= 110 * 1024 && cols <= 256) ? 2 : 1);
-  { const char* e_ = getenv("IEA_TC2_OCC"); if (e_ && occ == 3 && atoi(e_) == 2) occ = 2; }  // profiling switch
-  p.occ = occ;
-  const int cap = sms * occ;
+  const int occ = (cpr == 2 && smem <= 72 * 1024 && cols <= 128) ? 3 : ((cpr <= 4 && smem <= 110 * 1024 && cols <= 256) ? 2 : 1);
+  const int cap = sm_count() * occ;
   grid = p.n_tiles < cap ? p.n_tiles : cap;
-  smem_out = smem; cpr_out = cpr; is3_out = is3;
+  smem_out = smem; cpr_out = cpr; is3_out = is3; occ_out = occ;
   return 0;
 }
 static int tc2_grid(const iea_conv_desc* d) {
-  tc2::Params p; int grid = 0, cpr; uint32_t smem; bool is3;
-  if (tc2_prepare(d, p, grid, smem, cpr, is3)) return 0;
+  tc2::Params p; int grid = 0, cpr, occ; uint32_t smem; bool is3;
+  if (tc2_prepare(d, p, grid, smem, cpr, is3, occ)) return 0;
   return grid;
 }
 
 int iea_conv_fprop_tc2(const iea_conv_desc* d, cudaStream_t s) {
-  tc2::Params p; int grid = 0, cpr; uint32_t smem; bool is3;
-  int rc0 = tc2_prepare(d, p, grid, smem, cpr, is3);
+  tc2::Params p; int grid = 0, cpr, occ; uint32_t smem; bool is3;
+  int rc0 = tc2_prepare(d, p, grid, smem, cpr, is3, occ);
   if (rc0) return rc0;
   auto launch = [&](auto kern) -> int {
     IEA_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
@@ -1057,26 +980,20 @@ int iea_conv_fprop_tc2(const iea_conv_desc* d, cudaStream_t s) {
   };
   const int leanb = iea_conv_tc2_lean(d);
   const int tpe_ = tc2_tiles_per_event(d);
-  p.fd_tpe = tc2::make_fastdiv(tpe_ > 0 ? tpe_ : 1);
+  p.fd_tpe = tc::make_fastdiv(tpe_ > 0 ? tpe_ : 1);
   int rc = -2;
-  const int ko = cpr == 2 ? (p.occ == 3 ? 3 : 2) : (cpr == 4 ? 2 : 1);  // launch-bound variant of the kernel
-#define IEA_TC2_LAUNCH(C_, I_, L_, O_) \
+  const int ko = cpr == 2 ? (occ == 3 ? 3 : 2) : (cpr == 4 ? 2 : 1);  // launch-bound variant of the kernel
+#define TC2_LAUNCH(C_, I_, L_, O_) \
   if (cpr == C_ && is3 == I_ && leanb == L_ && ko == O_) rc = launch(tc2::conv_tc2_kernel<C_, I_, L_, O_>);
-  IEA_TC2_LAUNCH(2, true, 0, 3) IEA_TC2_LAUNCH(2, true, 1, 3) IEA_TC2_LAUNCH(2, true, 2, 3)
-  IEA_TC2_LAUNCH(2, true, 0, 2) IEA_TC2_LAUNCH(2, true, 1, 2) IEA_TC2_LAUNCH(2, true, 2, 2)
-  IEA_TC2_LAUNCH(4, true, 0, 2) IEA_TC2_LAUNCH(4, true, 1, 2) IEA_TC2_LAUNCH(4, true, 2, 2)
-  IEA_TC2_LAUNCH(8, true, 0, 1) IEA_TC2_LAUNCH(8, true, 1, 1) IEA_TC2_LAUNCH(8, true, 2, 1)
-  IEA_TC2_LAUNCH(2, false, 0, 3) IEA_TC2_LAUNCH(2, false, 1, 3) IEA_TC2_LAUNCH(2, false, 2, 3)
-  IEA_TC2_LAUNCH(2, false, 0, 2) IEA_TC2_LAUNCH(2, false, 1, 2) IEA_TC2_LAUNCH(2, false, 2, 2)
-  IEA_TC2_LAUNCH(4, false, 0, 2) IEA_TC2_LAUNCH(4, false, 1, 2) IEA_TC2_LAUNCH(4, false, 2, 2)
-  IEA_TC2_LAUNCH(8, false, 0, 1) IEA_TC2_LAUNCH(8, false, 1, 1) IEA_TC2_LAUNCH(8, false, 2, 1)
-#undef IEA_TC2_LAUNCH
+  TC2_LAUNCH(2, true, 0, 3) TC2_LAUNCH(2, true, 1, 3) TC2_LAUNCH(2, true, 2, 3)
+  TC2_LAUNCH(2, true, 0, 2) TC2_LAUNCH(2, true, 1, 2) TC2_LAUNCH(2, true, 2, 2)
+  TC2_LAUNCH(4, true, 0, 2) TC2_LAUNCH(4, true, 1, 2) TC2_LAUNCH(4, true, 2, 2)
+  TC2_LAUNCH(8, true, 0, 1) TC2_LAUNCH(8, true, 1, 1) TC2_LAUNCH(8, true, 2, 1)
+  TC2_LAUNCH(2, false, 0, 3) TC2_LAUNCH(2, false, 1, 3) TC2_LAUNCH(2, false, 2, 3)
+  TC2_LAUNCH(2, false, 0, 2) TC2_LAUNCH(2, false, 1, 2) TC2_LAUNCH(2, false, 2, 2)
+  TC2_LAUNCH(4, false, 0, 2) TC2_LAUNCH(4, false, 1, 2) TC2_LAUNCH(4, false, 2, 2)
+  TC2_LAUNCH(8, false, 0, 1) TC2_LAUNCH(8, false, 1, 1) TC2_LAUNCH(8, false, 2, 1)
+#undef TC2_LAUNCH
   if (rc) return rc;
   return check_launch("iea_conv_fprop(tcgen05 resident)");
 }
-
-#ifdef IEA_TC2_TRACE
-extern "C" int iea_debug_tc2_trace(long long* out) {
-  return (int)cudaMemcpyFromSymbol(out, tc2::g_trace, sizeof(long long) * 8 * 512);
-}
-#endif

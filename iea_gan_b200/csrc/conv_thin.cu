@@ -47,22 +47,6 @@ struct Geo {
   static constexpr uint32_t STAGE = (CPR * PLANE + 127) / 128 * 128;
 };
 
-#ifdef IEA_THIN_TRACE
-// pipeline trace of CTA 0 (profiling builds only): clock64 stamps per role and macro tile
-__device__ long long g_trace[8][512];
-#define TRACE(slot, idx) do { if (blockIdx.x == 0 && (idx) < 512) g_trace[slot][idx] = clock64(); } while (0)
-#else
-#define TRACE(slot, idx) do { } while (0)
-#endif
-
-// ablation switches of the profiling builds (-DIEA_THIN_DBG: IEA_TC2_DBG bits 1 no prologue transform, 2 no MMA,
-// 4 no output stores, 8 no statistics, 16 no loads); compiled out of the product kernel
-#ifdef IEA_THIN_DBG
-#define DBG(bit) (p.dbg & (bit))
-#else
-#define DBG(bit) 0
-#endif
-
 struct Params {
   iea_conv_desc d;
   const bf16* wtc;
@@ -71,8 +55,9 @@ struct Params {
   int n_macro;            // macro tiles
   int mtw, mth;           // macro tiles per image row / per image column (1x1: per image / 1)
   int hs, ws;             // stored input resolution
-  int stages, depth, dbg;
+  int stages;
   uint32_t w_bytes, stage_off, misc_off, bar_off, tmem_cols, tst_off, res_off, res_slot;  // tst_off: output staging of the TMA-store epilogue; res_off / res_slot: its residual ring
+  int depth;              // (behind the uint32_t block, which stays 8-byte aligned: pairs of it load as one 64-bit constant)
 };
 
 struct Pos { int n, th, tw; };
@@ -88,35 +73,11 @@ __device__ __forceinline__ void pos_next(const Params& p, Pos& c) {
   if (++c.tw == p.mtw) { c.tw = 0; if (++c.th == p.mth) { c.th = 0; ++c.n; } }
 }
 
-__device__ __forceinline__ float2 ffma2(float2 a, float2 b, float2 c) {
-  float2 r;
-  asm("fma.rn.f32x2 %0, %1, %2, %3;" : "=l"(reinterpret_cast<unsigned long long&>(r))
-      : "l"(reinterpret_cast<unsigned long long&>(a)), "l"(reinterpret_cast<unsigned long long&>(b)),
-        "l"(reinterpret_cast<unsigned long long&>(c)));
-  return r;
-}
-__device__ __forceinline__ float2 fadd2(float2 a, float2 b) {
-  float2 r;
-  asm("add.rn.f32x2 %0, %1, %2;" : "=l"(reinterpret_cast<unsigned long long&>(r))
-      : "l"(reinterpret_cast<unsigned long long&>(a)), "l"(reinterpret_cast<unsigned long long&>(b)));
-  return r;
-}
-__device__ __forceinline__ float2 bf2_to_f2(uint32_t w) {
-  return make_float2(__uint_as_float(w << 16), __uint_as_float(w & 0xFFFF0000u));
-}
 __device__ __forceinline__ bool elect_one() {
   uint32_t pred;
   asm volatile("{ .reg .pred P; elect.sync _|P, 0xffffffff; selp.u32 %0, 1, 0, P; }" : "=r"(pred));
   return pred != 0;
 }
-__device__ __forceinline__ void tmem_ld16_issue(uint32_t taddr, uint32_t* r) {
-  asm volatile(
-      "tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15}, [%16];"
-      : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]), "=r"(r[8]),
-        "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15])
-      : "r"(taddr));
-}
-__device__ __forceinline__ void tmem_ld_wait() { asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory"); }
 
 // EPI: epilogue flavour, fixed at compile time so that each is straight-line code (run-time flags made the
 // compiler shuffle the 16 accumulator registers at every merge point: ~200 instructions per 128x16 block
@@ -159,13 +120,9 @@ __global__ void __launch_bounds__(THREADS, 1) conv_thin_kernel(const __grid_cons
     mbar_init(w_bar, 1);
     if (TMA) for (int s = 0; s < S; ++s) mbar_init(land0 + 8 * s, 1);
     if (EPI == 3) for (int i = 0; i < 2 * RES_RING; ++i) mbar_init(bar0 + 24u * S + 80 + 8 * i, 1);  // residual ring: TMA landing
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    fence_mbar_init();
   }
-  if (warp == 0) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)),
-                 "r"(p.tmem_cols));
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;");
-  }
+  if (warp == 0) tmem_alloc(smem_u32(tmem_slot), p.tmem_cols);
   tc_fence_before();
   __syncthreads();
   tc_fence_after();
@@ -237,7 +194,6 @@ __global__ void __launch_bounds__(THREADS, 1) conv_thin_kernel(const __grid_cons
     };
     auto issue = [&](const Cur& c) {
       mbar_wait(empty0 + 8 * c.s, c.ph ^ 1);
-      if (DBG(16)) return;
       int64_t base;
       if (IS3) base = ((int64_t)(c.c.n * p.hs + ((c.c.th * 16) >> sh_)) * p.ws + ((c.c.tw * (8 * MT)) >> sh_)) * d.x_ld;
       else base = (int64_t)(g0 + c.t) * (BM * MT) * d.x_ld;
@@ -247,14 +203,13 @@ __global__ void __launch_bounds__(THREADS, 1) conv_thin_kernel(const __grid_cons
       if (pad == 0) {
 #pragma unroll
         for (int i = 0; i < NS; ++i)
-          if (i < NS - 1 || (m_valid >> i & 1))
-            asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(a + soff[i]), "l"(bp + goff[i]) : "memory");
+          if (i < NS - 1 || (m_valid >> i & 1)) cp16(a + soff[i], bp + goff[i]);
       } else {
 #pragma unroll
         for (int i = 0; i < NS; ++i) {
           if (!(m_valid >> i & 1)) continue;
           if (pad >> i & 1) asm volatile("st.shared.v4.b32 [%0], {%1,%1,%1,%1};" ::"r"(a + soff[i]), "r"(0) : "memory");
-          else asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(a + soff[i]), "l"(bp + goff[i]) : "memory");
+          else cp16(a + soff[i], bp + goff[i]);
         }
       }
     };
@@ -290,7 +245,7 @@ __global__ void __launch_bounds__(THREADS, 1) conv_thin_kernel(const __grid_cons
         bulk_g2s(sbase + off, (const uint8_t*)p.wtc + off, nb, w_bar);
       }
     }
-    constexpr uint32_t idesc = (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(BN >> 3) << 17) | ((uint32_t)(BM >> 4) << 24);
+    constexpr uint32_t ID = idesc(BN, false, false);
     constexpr uint32_t LBO_B = BN * 16;
     const uint64_t da_base = make_desc(sbase + p.stage_off, PLANE, IS3 ? PW * 16 : 128);
     const uint64_t db_base = make_desc(sbase, LBO_B, 128);
@@ -300,7 +255,6 @@ __global__ void __launch_bounds__(THREADS, 1) conv_thin_kernel(const __grid_cons
       mbar_wait(tempty0 + 8 * ab, aph ^ 1);
       mbar_wait(full0 + 8 * s, ph);
       tc_fence_after();
-      if (pt == 0) TRACE(3, t);
       if (elect_one()) {
         const uint32_t a16 = s * (STAGE >> 4);
         const uint32_t tacc = tmem_base + ab * (MT * BN);
@@ -311,7 +265,7 @@ __global__ void __launch_bounds__(THREADS, 1) conv_thin_kernel(const __grid_cons
             for (int j = 0; j < CPR / 2; ++j) {
               const uint32_t a_off = a16 + (IS3 ? sb * 8 + (tap / 3) * PW + (tap % 3) : sb * BM) + 2 * j * (PLANE >> 4);
               const uint32_t b_off = (uint32_t)((tap * CPR + 2 * j) * (LBO_B >> 4));
-              if (!DBG(2)) tc_mma(tacc + sb * BN, da_base + a_off, db_base + b_off, idesc, (tap > 0 || j > 0) ? 1u : 0u);
+              tc_mma(tacc + sb * BN, da_base + a_off, db_base + b_off, ID, (tap > 0 || j > 0) ? 1u : 0u);
             }
           }
         }
@@ -319,7 +273,6 @@ __global__ void __launch_bounds__(THREADS, 1) conv_thin_kernel(const __grid_cons
         tc_commit(tfull0 + 8 * ab);
       }
       __syncwarp();
-      if (pt == 0) TRACE(4, t);
     };
 
     Cur ci, ct;
@@ -331,7 +284,7 @@ __global__ void __launch_bounds__(THREADS, 1) conv_thin_kernel(const __grid_cons
         else if (pt == 0) issue_tma(ci);
         cur_next(ci);
       }
-      if (!TMA) asm volatile("cp.async.commit_group;" ::: "memory");
+      if (!TMA) cp_async_commit();
     }
     __nv_bfloat162 sc2[4], sh2[4];
     const __nv_bfloat162 zero2 = __floats2bfloat162_rn(0.f, 0.f);
@@ -343,15 +296,14 @@ __global__ void __launch_bounds__(THREADS, 1) conv_thin_kernel(const __grid_cons
         cur_next(ci);
       }
       if (!TMA) {
-        asm volatile("cp.async.commit_group;" ::: "memory");
-        if (D == 2) asm volatile("cp.async.wait_group 1;" ::: "memory");
-        else if (D == 3) asm volatile("cp.async.wait_group 2;" ::: "memory");
-        else asm volatile("cp.async.wait_group 3;" ::: "memory");
+        cp_async_commit();
+        if (D == 2) cp_async_wait<1>();
+        else if (D == 3) cp_async_wait<2>();
+        else cp_async_wait<3>();
       } else {
         mbar_wait(land0 + 8 * ct.s, ct.ph);  // the boxes of this macro tile have landed
       }
-      if (pt == 0) TRACE(0, ct.t);
-      if ((affine || relu) && !DBG(1)) {  // fused prologue, in place on the chunks this thread copied
+      if (affine || relu) {  // fused prologue, in place on the chunks this thread copied
         if (affine && ct.c.n != ss_n) {
           ss_n = ct.c.n;
           const int64_t si = (d.in_bcast ? 0 : (int64_t)ss_n * d.cin) + cc * 8;
@@ -392,15 +344,13 @@ __global__ void __launch_bounds__(THREADS, 1) conv_thin_kernel(const __grid_cons
             if (i0 + i < NS && (live >> (i0 + i) & 1)) *reinterpret_cast<uint4*>(a + soff[i0 + i]) = v[i];
         }
       }
-      if (pt == 0) TRACE(1, ct.t);
       fence_async_smem();
       __syncwarp();
       if (lane == 0) mbar_arrive(full0 + 8 * ct.s);
-      if (pt == 0) TRACE(2, ct.t);
       if (pw < NI) mma_item(ct.t, ct.s, ct.ph);
       cur_next(ct);
     }
-    if (!TMA) asm volatile("cp.async.wait_group 0;" ::: "memory");
+    if (!TMA) cp_async_wait<0>();
   } else {
     // ===================== epilogue: two groups of 4 warps, alternate macro tiles; one pixel per thread =====================
     const int grp = (warp - 8) >> 2;
@@ -537,10 +487,8 @@ __global__ void __launch_bounds__(THREADS, 1) conv_thin_kernel(const __grid_cons
 #pragma unroll
         for (int u = 0; u < (NB == 1 ? (MT < 2 ? MT : 2) : 1); ++u) res_prefetch(m0 + u * BM);
       }
-      if (et == 0) TRACE(5, t);
       mbar_wait(tfull0 + 8 * ab, aph);
       tc_fence_after();
-      if (et == 0) TRACE(6, t);
       // TMEM -> registers in batches of GRP sub-tiles: the loads are issued back to back and waited for
       // once, and the sub-tiles of a batch are independent instruction streams
       constexpr int GRP = NB == 1 ? (MT < 2 ? MT : 2) : 1;
@@ -651,11 +599,11 @@ __global__ void __launch_bounds__(THREADS, 1) conv_thin_kernel(const __grid_cons
               uint8_t* row_ = st_ptr + (st_cnt & 1) * ST_IMG + et * RB;
               *reinterpret_cast<uint4*>(row_ + (((2 * cb) ^ st_sw) << 4)) = make_uint4(o[0], o[1], o[2], o[3]);
               *reinterpret_cast<uint4*>(row_ + (((2 * cb + 1) ^ st_sw) << 4)) = make_uint4(o[4], o[5], o[6], o[7]);
-            } else if (!DBG(4)) {
+            } else {
               yp[0] = make_uint4(o[0], o[1], o[2], o[3]);
               yp[1] = make_uint4(o[4], o[5], o[6], o[7]);
             }
-            if (has_stats && !DBG(8)) {
+            if (has_stats) {
 #pragma unroll
               for (int j = 0; j < 8; ++j) { s1[cb * 8 + j] = fadd2(s1[cb * 8 + j], v[j]); s2[cb * 8 + j] = ffma2(v[j], v[j], s2[cb * 8 + j]); }
             }
@@ -678,7 +626,6 @@ __global__ void __launch_bounds__(THREADS, 1) conv_thin_kernel(const __grid_cons
       tc_fence_before();
       __syncwarp();
       if (lane == 0) mbar_arrive(tempty0 + 8 * ab);
-      if (et == 0) TRACE(7, t);
     }
     if (has_stats && any) flush(ev);
     if (TST && et == 0) asm volatile("cp.async.bulk.wait_group 0;" ::: "memory");
@@ -687,7 +634,7 @@ __global__ void __launch_bounds__(THREADS, 1) conv_thin_kernel(const __grid_cons
   __syncthreads();
   if (warp == 0) {
     tc_fence_after();
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(p.tmem_cols));
+    tmem_free(tmem_base, p.tmem_cols);
   }
 }
 
@@ -796,10 +743,9 @@ static int thin_prepare(const iea_conv_desc* d, thin::Params& p, int& grid, uint
   using G = thin::Geo<CPR, IS3, MT, TMA>;
   p.d = *d;
   p.wtc = (const bf16*)d->wpack_tc;
-  { const char* e_ = getenv("IEA_TC2_DBG"); p.dbg = e_ ? atoi(e_) : 0; }  // profiling ablations only
   p.M = (int)(d->n * (int64_t)d->h * d->w);
-  p.hs = d->in_mode == IEA_IN_UP2 ? d->h / 2 : d->h;
-  p.ws = d->in_mode == IEA_IN_UP2 ? d->w / 2 : d->w;
+  p.hs = stored_res(*d, d->h);
+  p.ws = stored_res(*d, d->w);
   const int hw = d->h * d->w;
   if (IS3) {
     p.mtw = d->w / (8 * MT); p.mth = d->h / 16;
@@ -831,14 +777,11 @@ static int thin_prepare(const iea_conv_desc* d, thin::Params& p, int& grid, uint
   p.misc_off = tst ? p.res_off + ring_bytes : p.stage_off + stages * G::STAGE;
   p.bar_off = (p.misc_off + misc + 15) / 16 * 16;
   smem = p.bar_off + 512;  // barriers: full, empty, landing (8 B x stages each), 2 x 4 accumulator, weights; TMEM slot
-  uint32_t cols = 32;
-  while (cols < (uint32_t)(4 * MT * cout_e)) cols <<= 1;
+  const uint32_t cols = tmem_cols_for(4 * MT * cout_e);
   p.tmem_cols = cols;
   IEA_CHECK_ARG(smem <= 220 * 1024 && cols <= 512, "iea_conv_fprop(tcgen05 thin): tile does not fit (cin=%d cout=%d k=%d)",
                 d->cin, d->cout, d->ksize);
-  int dev = 0, sms = 148;
-  cudaGetDevice(&dev);
-  cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+  const int sms = sm_count();
   grid = p.n_macro < sms ? p.n_macro : sms;
   return 0;
 }
@@ -911,9 +854,3 @@ int iea_conv_thin_stats_slots(const iea_conv_desc* d) {
   if (thin_dispatch(d, nullptr, &grid)) return 0;
   return 2 * grid;
 }
-
-#ifdef IEA_THIN_TRACE
-extern "C" int iea_debug_thin_trace(long long* out) {
-  return (int)cudaMemcpyFromSymbol(out, thin::g_trace, sizeof(long long) * 8 * 512);
-}
-#endif

@@ -152,8 +152,7 @@ __global__ void __launch_bounds__(256) wgrad_mma_kernel(const Params p) {
         const uint32_t lo = (uint32_t)__bfloat16_as_ushort(__float2bfloat16_rn(v));
         asm volatile("st.shared.v4.b32 [%0], {%1,%2,%2,%2};" ::"r"(dst), "r"(lo), "r"(0) : "memory");
       } else {
-        const bf16* src = (const bf16*)d.x + pix * d.x_ld + ca0 + c * 8;
-        asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(dst), "l"(src) : "memory");
+        cp16(dst, (const bf16*)d.x + pix * d.x_ld + ca0 + c * 8);
       }
     }
     // ---- output-gradient tile: 128 pixels x cout, pixel r = (r>>3, r&7) inside a 16x8 tile
@@ -176,15 +175,14 @@ __global__ void __launch_bounds__(256) wgrad_mma_kernel(const Params p) {
           }
         asm volatile("st.shared.v4.b32 [%0], {%1,%2,%3,%4};" ::"r"(dst), "r"(w4[0]), "r"(w4[1]), "r"(w4[2]), "r"(w4[3]) : "memory");
       } else {
-        const bf16* src = (const bf16*)p.g + m * p.g_ld + cg0 + c * 8;
-        asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(dst), "l"(src) : "memory");
+        cp16(dst, (const bf16*)p.g + m * p.g_ld + cg0 + c * 8);
       }
     }
   };
 
   for (int k = 0; k < D - 1; ++k) {
     if (k < my_tiles) issue(k);
-    asm volatile("cp.async.commit_group;" ::: "memory");
+    cp_async_commit();
   }
   // warp -> (output block pairs, k-step group)
   const int nib = p.nib_l;  // 16-wide ci blocks of this CTA
@@ -196,12 +194,12 @@ __global__ void __launch_bounds__(256) wgrad_mma_kernel(const Params p) {
 
   for (int it = 0; it < my_tiles; ++it) {
     if (it + D - 1 < my_tiles) issue(it + D - 1);
-    asm volatile("cp.async.commit_group;" ::: "memory");
+    cp_async_commit();
     switch (D) {
-      case 2: asm volatile("cp.async.wait_group 1;" ::: "memory"); break;
-      case 3: asm volatile("cp.async.wait_group 2;" ::: "memory"); break;
-      case 4: asm volatile("cp.async.wait_group 3;" ::: "memory"); break;
-      default: asm volatile("cp.async.wait_group 0;" ::: "memory"); break;
+      case 2: cp_async_wait<1>(); break;
+      case 3: cp_async_wait<2>(); break;
+      case 4: cp_async_wait<3>(); break;
+      default: cp_async_wait<0>(); break;
     }
     const Origin o = tile_origin<IS3>(p, (int)blockIdx.x + it * (int)gridDim.x);
     const uint32_t s0 = sbase + (uint32_t)(it % p.stages) * p.stage_bytes;
@@ -263,7 +261,7 @@ __global__ void __launch_bounds__(256) wgrad_mma_kernel(const Params p) {
     }
     __syncthreads();  // the stage is overwritten by the cp.async of the next iteration
   }
-  asm volatile("cp.async.wait_group 0;" ::: "memory");
+  cp_async_wait<0>();
   // ---- fold the k-step groups of the CTA (fixed order), then one partial per CTA:
   //      gpart[blockIdx.x][cout][taps][cin]
   if (p.WP > 1) {  // NPAIR == 1 here; scratch [P][TAPS*8][32] floats re-uses the pipeline smem
@@ -420,11 +418,11 @@ __global__ void __launch_bounds__(256) wgrad3_kernel(const P3 p) {
     for (int i = 0; i < NSA; ++i) {
       if (!(m_valid >> i & 1)) continue;
       if (pad >> i & 1) asm volatile("st.shared.v4.b32 [%0], {%1,%1,%1,%1};" ::"r"(s0 + soa[i]), "r"(0) : "memory");
-      else asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(s0 + soa[i]), "l"(ap + goa[i]) : "memory");
+      else cp16(s0 + soa[i], ap + goa[i]);
     }
 #pragma unroll
     for (int i = 0; i < NSG; ++i)
-      asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(s0 + sog[i]), "l"(gp + gog[i]) : "memory");
+      cp16(s0 + sog[i], gp + gog[i]);
   };
 
   const int pair = warp % P, kg = warp / P;
@@ -442,7 +440,7 @@ __global__ void __launch_bounds__(256) wgrad3_kernel(const P3 p) {
 
   for (int k = 0; k < D - 1; ++k) {
     if (k < my_n) issue(k);
-    asm volatile("cp.async.commit_group;" ::: "memory");
+    cp_async_commit();
   }
   __nv_bfloat162 sc2[4], sh2[4];
   const __nv_bfloat162 zero2 = __floats2bfloat162_rn(0.f, 0.f);
@@ -450,9 +448,9 @@ __global__ void __launch_bounds__(256) wgrad3_kernel(const P3 p) {
   const int mat = lane >> 3, rr = lane & 7;
   for (int it = 0; it < my_n; ++it) {
     if (it + D - 1 < my_n) issue(it + D - 1);
-    asm volatile("cp.async.commit_group;" ::: "memory");
-    if (D == 2) asm volatile("cp.async.wait_group 1;" ::: "memory");
-    else asm volatile("cp.async.wait_group 2;" ::: "memory");
+    cp_async_commit();
+    if (D == 2) cp_async_wait<1>();
+    else cp_async_wait<2>();
     const uint32_t s0 = sbase + (uint32_t)(it % p.stages) * G::STAGE;
     if (affine || relu) {  // fused prologue, in place on the chunks this thread copied; padding stays zero
       const Pos c = pos_of((int)blockIdx.x + it * (int)gridDim.x);
@@ -506,7 +504,7 @@ __global__ void __launch_bounds__(256) wgrad3_kernel(const P3 p) {
     }
     __syncthreads();  // the stage is overwritten by the cp.async of the next iteration
   }
-  asm volatile("cp.async.wait_group 0;" ::: "memory");
+  cp_async_wait<0>();
   // ---- fold the k-step groups (fixed order), then one partial per CTA: gpart[blockIdx.x][cout][9][cin]
   if (WP > 1) {
     float* scr = reinterpret_cast<float*>(smem);  // [P][TAPS*8 + 4][32]
@@ -615,8 +613,8 @@ static int wgrad_mma_plan(const iea_conv_desc* d, int g_dtype, int g_ld, WgradPl
   if (P <= 8) WP = 8 / P; else npair = P / 8;
   p->d = *d;
   p->M = M;
-  p->hs = d->in_mode == IEA_IN_UP2 ? d->h / 2 : (d->in_mode == IEA_IN_POOL2 ? d->h * 2 : d->h);
-  p->ws = d->in_mode == IEA_IN_UP2 ? d->w / 2 : (d->in_mode == IEA_IN_POOL2 ? d->w * 2 : d->w);
+  p->hs = stored_res(*d, d->h);
+  p->ws = stored_res(*d, d->w);
   p->fd_w = wg::make_fastdiv(d->w); p->fd_h = wg::make_fastdiv(d->h);
   p->tiles_w = is3 ? (d->w + 7) / 8 : 1;    // edge tiles are masked (8x8 / 4x4 layers: one partly filled tile per image)
   p->tiles_h = is3 ? (d->h + 15) / 16 : 1;
@@ -637,9 +635,7 @@ static int wgrad_mma_plan(const iea_conv_desc* d, int g_dtype, int g_ld, WgradPl
   p->stages = stages;
   p->depth = stages >= 4 ? 3 : 2;
   p->P = P; p->WP = WP;
-  int dev = 0, sms = 148;
-  cudaGetDevice(&dev);
-  cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+  const int sms = sm_count();
   pl.smem = p->stages * p->stage_bytes;
   const int occ = pl.smem <= 100 * 1024 ? 2 : 1;
   if (WP > 1 && pl.smem < (uint32_t)(P * (taps * 8 + 4) * 32 * 4)) pl.smem = P * (taps * 8 + 4) * 32 * 4;  // fold scratch
@@ -685,8 +681,8 @@ template <int CPA, int CPG, int MT, bool IS3>
 static int wgrad3_setup(const iea_conv_desc* d, wg::P3& p, int& grid, uint32_t& smem) {
   using G = wg::G3<CPA, CPG, MT, IS3>;
   p.d = *d;
-  p.hs = d->in_mode == IEA_IN_UP2 ? d->h / 2 : d->h;
-  p.ws = d->in_mode == IEA_IN_UP2 ? d->w / 2 : d->w;
+  p.hs = stored_res(*d, d->h);
+  p.ws = stored_res(*d, d->w);
   if (IS3) { p.mtw = d->w / (8 * MT); p.mth = d->h / 16; }
   else { p.mtw = (int)(((int64_t)d->h * d->w) / (128 * MT)); p.mth = 1; }  // macro tiles per image
   p.n_macro = (int)(d->n * (int64_t)p.mtw * p.mth);
@@ -696,9 +692,7 @@ static int wgrad3_setup(const iea_conv_desc* d, wg::P3& p, int& grid, uint32_t& 
   smem = p.stages * G::STAGE;
   constexpr uint32_t fold = (uint32_t)((CPA / 2) * (CPG / 2)) * ((IS3 ? 72 : 8) + 4) * 32 * 4;
   if (smem < fold) smem = fold;
-  int dev = 0, sms = 148;
-  cudaGetDevice(&dev);
-  cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+  const int sms = sm_count();
   const int occ = smem <= 110 * 1024 ? 2 : 1;
   grid = p.n_macro < sms * occ ? p.n_macro : sms * occ;
   return 0;

@@ -37,9 +37,6 @@ struct Params {
   uint32_t g_bytes, x_bytes, buf_bytes, bar_off, tmem_cols;
 };
 
-__host__ __device__ constexpr uint32_t idesc_mn(int n) {  // D fp32, A / B bf16, both MN-major, M = 128
-  return (1u << 4) | (1u << 7) | (1u << 10) | (1u << 15) | (1u << 16) | ((uint32_t)(n >> 3) << 17) | ((uint32_t)(128 >> 4) << 24);
-}
 __device__ __forceinline__ uint64_t desc_mn(uint32_t addr) { return make_desc(addr, 128, PL); }
 
 __global__ void __launch_bounds__(THREADS, 1) wgrad_tc_kernel(const Params p) {
@@ -52,12 +49,9 @@ __global__ void __launch_bounds__(THREADS, 1) wgrad_tc_kernel(const Params p) {
   if (tid == 0) {
     mbar_init(bar0, 1);
     mbar_init(bar0 + 8, 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    fence_mbar_init();
   }
-  if (warp == 0) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)), "r"(p.tmem_cols));
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;");
-  }
+  if (warp == 0) tmem_alloc(smem_u32(tmem_slot), p.tmem_cols);
   tc_fence_before();
   __syncthreads();
   tc_fence_after();
@@ -135,7 +129,7 @@ __global__ void __launch_bounds__(THREADS, 1) wgrad_tc_kernel(const Params p) {
     if (tid == 0) {
       tc_fence_after();
       const uint32_t a0 = sbase + b * p.buf_bytes;
-      const uint32_t id = idesc_mn(p.nb);
+      const uint32_t id = idesc(p.nb, true, true);
       for (int s = 0; s < nslot; ++s) {
         const uint32_t x0 = a0 + p.g_bytes + s * p.x_bytes;
 #pragma unroll
@@ -173,7 +167,7 @@ __global__ void __launch_bounds__(THREADS, 1) wgrad_tc_kernel(const Params p) {
   }
   tc_fence_before();
   __syncthreads();
-  if (warp == 0) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem), "r"(p.tmem_cols));
+  if (warp == 0) tmem_free(tmem, p.tmem_cols);
 }
 
 static bool plan(const iea_conv_desc* d, int g_dtype, int g_ld, Params* p) {
@@ -186,8 +180,8 @@ static bool plan(const iea_conv_desc* d, int g_dtype, int g_ld, Params* p) {
   if (d->in_scale && (!aligned16(d->in_scale) || !aligned16(d->in_shift) || d->cin % 4)) return false;
   p->d = *d;
   p->M = M;
-  p->hs = d->in_mode == IEA_IN_UP2 ? d->h / 2 : (d->in_mode == IEA_IN_POOL2 ? d->h * 2 : d->h);
-  p->ws = d->in_mode == IEA_IN_UP2 ? d->w / 2 : (d->in_mode == IEA_IN_POOL2 ? d->w * 2 : d->w);
+  p->hs = stored_res(*d, d->h);
+  p->ws = stored_res(*d, d->w);
   p->nb = d->cin < 128 ? d->cin : 128;
   p->cprx = p->nb / 8;
   p->cin_blocks = d->cin / p->nb;

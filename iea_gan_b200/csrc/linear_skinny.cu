@@ -129,9 +129,7 @@ int iea_linear_skinny_ok(const iea_conv_desc* d) {
 int iea_linear_skinny(const iea_conv_desc* d, cudaStream_t s) {
   const int M = (int)d->n;
   const int tiles = cdiv(M, lsk::BM) * cdiv(d->cout, lsk::BN);
-  int dev = 0, sms = 148;
-  cudaGetDevice(&dev);
-  cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+  const int sms = sm_count();
   int split = 1;  // cluster size: enough CTAs to fill the chip, at least 128 K elements per CTA
   while (split < 8 && tiles * split < 2 * sms && d->cin / (split * 2) >= 128) split *= 2;
   int kper = cdiv(d->cin, split);

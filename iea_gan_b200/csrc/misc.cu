@@ -51,26 +51,15 @@ __global__ void axpby_kernel(const void* a, int adt, float alpha, const void* b,
 }
 
 // 8 bf16 per thread and access (16 bytes): the scalar forms below move 2 bytes per load and ran at 1.4 TB/s
-__device__ __forceinline__ void bf8_unpack(const uint4& q, float* f) {
-  const uint32_t w[4] = {q.x, q.y, q.z, q.w};
-#pragma unroll
-  for (int i = 0; i < 4; ++i) { f[2 * i] = __uint_as_float(w[i] << 16); f[2 * i + 1] = __uint_as_float(w[i] & 0xFFFF0000u); }
-}
-__device__ __forceinline__ uint4 bf8_pack(const float* f) {
-  uint32_t w[4];
-#pragma unroll
-  for (int i = 0; i < 4; ++i) { __nv_bfloat162 t = __floats2bfloat162_rn(f[2 * i], f[2 * i + 1]); w[i] = *reinterpret_cast<uint32_t*>(&t); }
-  return make_uint4(w[0], w[1], w[2], w[3]);
-}
 __global__ void __launch_bounds__(256) gamma_res_vec_kernel(const uint4* o, const uint4* x, const float* gamma, uint4* y,
                                                             int64_t n8) {
   const float g = gamma[0];
   for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n8; i += (int64_t)gridDim.x * blockDim.x) {
     float a[8], b[8];
-    bf8_unpack(o[i], a); bf8_unpack(x[i], b);
+    unpack8(o[i], a); unpack8(x[i], b);
 #pragma unroll
     for (int j = 0; j < 8; ++j) a[j] = fmaf(g, a[j], b[j]);
-    y[i] = bf8_pack(a);
+    y[i] = pack8(a);
   }
 }
 __global__ void __launch_bounds__(256) gamma_res_bwd_vec_kernel(const uint4* dy, const uint4* o, const float* gamma,
@@ -80,10 +69,10 @@ __global__ void __launch_bounds__(256) gamma_res_bwd_vec_kernel(const uint4* dy,
   float acc = 0.f;
   for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n8; i += (int64_t)gridDim.x * blockDim.x) {
     float d[8], v[8];
-    bf8_unpack(dy[i], d); bf8_unpack(o[i], v);
+    unpack8(dy[i], d); unpack8(o[i], v);
 #pragma unroll
     for (int j = 0; j < 8; ++j) { acc = fmaf(d[j], v[j], acc); d[j] *= g; }
-    d_o[i] = bf8_pack(d);
+    d_o[i] = pack8(d);
   }
   acc = block_sum(acc, red);
   if (threadIdx.x == 0) part[blockIdx.x] = acc;
@@ -92,16 +81,16 @@ __global__ void __launch_bounds__(256) axpby_bf16_vec_kernel(const uint4* a, flo
                                                              uint4* y, int64_t n8) {
   for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n8; i += (int64_t)gridDim.x * blockDim.x) {
     float u[8], v[8];
-    bf8_unpack(a[i], u);
+    unpack8(a[i], u);
     if (b) {
-      bf8_unpack(b[i], v);
+      unpack8(b[i], v);
 #pragma unroll
       for (int j = 0; j < 8; ++j) u[j] = fmaf(beta, v[j], alpha * u[j]);
     } else {
 #pragma unroll
       for (int j = 0; j < 8; ++j) u[j] *= alpha;
     }
-    y[i] = bf8_pack(u);
+    y[i] = pack8(u);
   }
 }
 __device__ __host__ inline bool al16_3(const void* a, const void* b, const void* c) {

@@ -1,5 +1,5 @@
-// tc_common.cuh -- PTX wrappers shared by the tcgen05 convolution kernels (mbarrier, TMA bulk copy,
-// tcgen05 alloc/mma/commit/ld, UMMA shared-memory descriptors) and the fused-prologue chunk loader.
+// tc_common.cuh -- PTX wrappers shared by the tcgen05 kernels (mbarrier, TMA bulk copy, tcgen05
+// alloc/mma/commit/ld, UMMA instruction and shared-memory descriptors) and the fused-prologue chunk loader.
 #pragma once
 #include "common.cuh"
 
@@ -11,6 +11,8 @@ __device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)_
 __device__ __forceinline__ void mbar_init(uint32_t bar, uint32_t count) {
   asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(bar), "r"(count));
 }
+// makes the barrier initialisation visible to the async proxy (TMA, tcgen05.commit) before any use
+__device__ __forceinline__ void fence_mbar_init() { asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory"); }
 __device__ __forceinline__ void mbar_arrive(uint32_t bar) {
   asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(bar) : "memory");
 }
@@ -50,6 +52,12 @@ __device__ __forceinline__ void tc_mma(uint32_t tmem_c, uint64_t da, uint64_t db
       "l"(da), "l"(db), "r"(idesc), "r"(acc)
       : "memory");
 }
+// UMMA instruction descriptor: bf16 A and B, fp32 accumulator, M = 128, N = n; a_mn / b_mn: the operand is
+// MN-major (reduction along its rows) instead of K-major
+__host__ __device__ constexpr uint32_t idesc(int n, bool a_mn, bool b_mn) {
+  return (1u << 4) | (1u << 7) | (1u << 10) | ((a_mn ? 1u : 0u) << 15) | ((b_mn ? 1u : 0u) << 16) |
+         ((uint32_t)(n >> 3) << 17) | ((uint32_t)(128 >> 4) << 24);
+}
 __device__ __forceinline__ uint64_t make_desc(uint32_t addr, uint32_t lbo, uint32_t sbo) {
   uint64_t d = 0;
   d |= (uint64_t)((addr >> 4) & 0x3FFF);
@@ -58,34 +66,33 @@ __device__ __forceinline__ uint64_t make_desc(uint32_t addr, uint32_t lbo, uint3
   d |= (uint64_t)1 << 46;  // descriptor version for sm_100
   return d;                // layout_type = 0 (no swizzle), base_offset = 0
 }
-__device__ __forceinline__ void tmem_ld16(uint32_t taddr, float* v) {
-  uint32_t r[16];
+// tcgen05.ld of 16 accumulator columns of this warp's 32 lanes, split into issue and wait so that several loads
+// can be in flight before one wait
+__device__ __forceinline__ void tmem_ld16_issue(uint32_t taddr, uint32_t* r) {
   asm volatile(
       "tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15}, [%16];"
       : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]), "=r"(r[8]),
         "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15])
       : "r"(taddr));
-  asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+}
+__device__ __forceinline__ void tmem_ld_wait() { asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory"); }
+__device__ __forceinline__ void tmem_ld16(uint32_t taddr, float* v) {
+  uint32_t r[16];
+  tmem_ld16_issue(taddr, r);
+  tmem_ld_wait();
 #pragma unroll
   for (int i = 0; i < 16; ++i) v[i] = __uint_as_float(r[i]);
 }
+// one warp allocates `cols` TMEM columns (address written to shared memory at `slot`) and gives up the permit;
+// the same warp frees them at the end
+__device__ __forceinline__ void tmem_alloc(uint32_t slot, uint32_t cols) {
+  asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(slot), "r"(cols));
+  asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;");
+}
+__device__ __forceinline__ void tmem_free(uint32_t base, uint32_t cols) {
+  asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(base), "r"(cols));
+}
 __device__ __forceinline__ void bar_sync_epi() { asm volatile("bar.sync 1, 128;" ::: "memory"); }
-
-__device__ __forceinline__ void unpack8(const uint4& q, float* f) {
-  const uint32_t w[4] = {q.x, q.y, q.z, q.w};
-#pragma unroll
-  for (int i = 0; i < 4; ++i) {
-    f[2 * i] = __uint_as_float(w[i] << 16);
-    f[2 * i + 1] = __uint_as_float(w[i] & 0xFFFF0000u);
-  }
-}
-__device__ __forceinline__ uint32_t pack2(float a, float b) {
-  __nv_bfloat162 t = __floats2bfloat162_rn(a, b);
-  return *reinterpret_cast<uint32_t*>(&t);
-}
-__device__ __forceinline__ uint4 pack8(const float* f) {
-  return make_uint4(pack2(f[0], f[1]), pack2(f[2], f[3]), pack2(f[4], f[5]), pack2(f[6], f[7]));
-}
 
 // one 16-byte chunk (8 channels starting at ci) of T(x) at conv-resolution pixel (n, ih, iw)
 __device__ __forceinline__ uint4 load_chunk(const iea_conv_desc& d, int hs, int ws, int64_t n, int ih, int iw, int ci) {
@@ -153,6 +160,5 @@ __device__ __forceinline__ uint32_t fdiv(uint32_t n, const FastDiv& f) {
   const uint32_t t = __umulhi(n, f.mul);
   return (t + ((n - t) >> 1)) >> (f.shr - 1);
 }
-
 
 }  // namespace tc

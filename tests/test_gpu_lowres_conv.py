@@ -48,8 +48,9 @@ def _run(eng, variant, cin, cout, mode, relu, aff, resm, hw, n, stats):
             rh, rw = (h // 2, w // 2) if resm == 1 else (h, w)
             res = torch.randn(n, rh, rw, cout + 16, device=dev).bfloat16()
         g = torch.randn(n, h, w, cout, device=dev).bfloat16()
-        torch.cuda.synchronize()
-        with torch.profiler.profile(activities=[torch.profiler.ProfilerActivity.CUDA]) as prof:
+
+        def once():
+            m.bias.requires_grad_(True)
             tape = eng.Tape(True)
             xv = eng.Var(x)
             ss = eng.ScaleShift(scale, shift) if aff else None
@@ -59,6 +60,15 @@ def _run(eng, variant, cin, cout, mode, relu, aff, resm, hw, n, stats):
             yv.g = g
             m.bias.requires_grad_(False)
             tape.backward()
+            return xv, yv
+
+        # The layer runs twice, identically, inside the profiled region and the outputs are the second pass's.  Late
+        # in a long test process the profiler drops the first kernel records of each session (three per session in
+        # the full suite, none in a fresh process); at one image that is the whole forward and data gradient.
+        torch.cuda.synchronize()
+        with torch.profiler.profile(activities=[torch.profiler.ProfilerActivity.CUDA]) as prof:
+            once()
+            xv, yv = once()
             torch.cuda.synchronize()
         names = " ".join(e.key for e in prof.key_averages())
         st = yv.bn[0].clone() if (stats and yv.bn) else None

@@ -15,24 +15,29 @@ int iea_conv_tc2_stats_slots(const iea_conv_desc* d);
 int iea_conv_thin_ok(const iea_conv_desc* d);
 int iea_conv_fprop_thin(const iea_conv_desc* d, cudaStream_t s);
 int iea_conv_thin_stats_slots(const iea_conv_desc* d);
+int iea_conv_wide_ok(const iea_conv_desc* d);
+int iea_conv_fprop_wide(const iea_conv_desc* d, cudaStream_t s);
 int iea_conv_c1_fwd_ok(const iea_conv_desc* d);
 int iea_conv_c1_fwd(const iea_conv_desc* d, cudaStream_t s);
 int iea_linear_skinny_ok(const iea_conv_desc* d);
 int iea_linear_skinny(const iea_conv_desc* d, cudaStream_t s);
 
-enum class ConvKernel { generic, c1, skinny, thin, tc2, lowres, stream };
+enum class ConvKernel { generic, c1, skinny, thin, wide, tc2, lowres, stream };
 
-// auto: c1, then skinny, then the tcgen05 chain (thin -> tc2 -> lowres -> stream), else generic.  tcgen05 and
-// tc_stream run the tcgen05 chain only; tc_stream skips thin and lowres and takes the streaming kernel wherever
+// auto: c1, then skinny, then the tcgen05 chain (thin -> wide -> tc2 -> lowres -> stream), else generic.  tc2 routes
+// as auto but never picks wide (its shapes run on conv_tc2, the reference conv_wide is tested against).  tcgen05 and
+// tc_stream run the tcgen05 chain only; tc_stream skips thin, wide and lowres and takes the streaming kernel wherever
 // iea_conv_tc_ok accepts the shape.  Returns generic when tcgen05 does not accept the shape.
 static ConvKernel conv_route(const iea_conv_desc* d) {
   if (d->impl == IEA_IMPL_GENERIC) return ConvKernel::generic;
-  if (d->impl == IEA_IMPL_AUTO && iea_conv_c1_fwd_ok(d)) return ConvKernel::c1;
-  if (d->impl == IEA_IMPL_AUTO && iea_linear_skinny_ok(d)) return ConvKernel::skinny;
+  const bool auto_ = d->impl == IEA_IMPL_AUTO || d->impl == IEA_IMPL_TC2;
+  if (auto_ && iea_conv_c1_fwd_ok(d)) return ConvKernel::c1;
+  if (auto_ && iea_linear_skinny_ok(d)) return ConvKernel::skinny;
   const bool tc_ok = iea_conv_tc_ok(d), tc2_ok = iea_conv_tc2_ok(d);
   if (!tc_ok && !tc2_ok) return ConvKernel::generic;
   const bool force_stream = d->impl == IEA_IMPL_TC_STREAM;
   if (!force_stream && iea_conv_thin_ok(d)) return ConvKernel::thin;
+  if (!force_stream && d->impl != IEA_IMPL_TC2 && iea_conv_wide_ok(d)) return ConvKernel::wide;
   if ((!force_stream || !tc_ok) && tc2_ok) return ConvKernel::tc2;
   if (!force_stream && iea_conv_lowres_ok(d)) return ConvKernel::lowres;
   return ConvKernel::stream;
@@ -55,7 +60,7 @@ extern "C" int iea_conv_stats_slots(const iea_conv_desc* d) {
   switch (conv_route(d)) {
     case ConvKernel::thin: return iea_conv_thin_stats_slots(d);
     case ConvKernel::tc2: return iea_conv_tc2_stats_slots(d);
-    default: {  // one slot per 128-pixel tile
+    default: {  // one slot per 128-pixel tile (conv_wide and the staged conv_tc2 epilogue included)
       const int64_t px = 40ll * d->h * d->w;
       return (d->n % 40 == 0 && px % 128 == 0) ? (int)(px / 128) : 0;
     }
@@ -76,6 +81,7 @@ extern "C" int iea_conv_fprop(const iea_conv_desc* d, iea_stream_t stream) {
     case ConvKernel::c1: return iea_conv_c1_fwd(d, s);
     case ConvKernel::skinny: return iea_linear_skinny(d, s);
     case ConvKernel::thin: return iea_conv_fprop_thin(d, s);
+    case ConvKernel::wide: return iea_conv_fprop_wide(d, s);
     case ConvKernel::tc2: return iea_conv_fprop_tc2(d, s);
     case ConvKernel::lowres: return iea_conv_fprop_lowres(d, s);
     case ConvKernel::stream: return iea_conv_fprop_tc(d, s);

@@ -17,7 +17,6 @@
 // Shapes outside this envelope (pooled inputs, Cout > 32, Cin > 64, the 1-channel stem) stay on
 // conv_tc2.cu / conv_tc.cu.
 #include "tc_common.cuh"
-#include <cuda.h>
 #include <stdlib.h>
 #include <string.h>
 using namespace iea;
@@ -71,12 +70,6 @@ __device__ __forceinline__ Pos pos_of(const Params& p, int g) {
 }
 __device__ __forceinline__ void pos_next(const Params& p, Pos& c) {
   if (++c.tw == p.mtw) { c.tw = 0; if (++c.th == p.mth) { c.th = 0; ++c.n; } }
-}
-
-__device__ __forceinline__ bool elect_one() {
-  uint32_t pred;
-  asm volatile("{ .reg .pred P; elect.sync _|P, 0xffffffff; selp.u32 %0, 1, 0, P; }" : "=r"(pred));
-  return pred != 0;
 }
 
 // EPI: epilogue flavour, fixed at compile time so that each is straight-line code (run-time flags made the
@@ -677,23 +670,10 @@ int iea_conv_thin_ok(const iea_conv_desc* d) {
   return 1;
 }
 
-// ---- TMA tensor map of the input (driver entry point: the library does not link libcuda)
-typedef CUresult (*encode_tiled_fn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
-                                    const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
-                                    CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-static encode_tiled_fn tma_encoder() {
-  static encode_tiled_fn fn = nullptr;
-  if (!fn) {
-    void* p = nullptr;
-    cudaDriverEntryPointQueryResult q;
-    if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q) == cudaSuccess && q == cudaDriverEntryPointSuccess)
-      fn = (encode_tiled_fn)p;
-  }
-  return fn;
-}
+// ---- TMA tensor maps of the input, output and residual
 // output of a 1x1 layer as {cout channels, pixels}: boxes {cout, 128}, chunks swizzled inside the 64 / 32-byte rows
 static bool thin_tensor_map_y(const iea_conv_desc* d, CUtensorMap* tm) {
-  encode_tiled_fn enc = tma_encoder();
+  tc::encode_tiled_fn enc = tc::tma_encoder();
   if (!enc || d->y_dtype != IEA_BF16 || d->y_ld % 8 || ((uintptr_t)d->y & 15) || (d->cout != 16 && d->cout != 32)) return false;
   const cuuint64_t dims[2] = {(cuuint64_t)d->cout, (cuuint64_t)(d->n * (int64_t)d->h * d->w)};
   const cuuint64_t strides[1] = {(cuuint64_t)d->y_ld * 2};
@@ -705,7 +685,7 @@ static bool thin_tensor_map_y(const iea_conv_desc* d, CUtensorMap* tm) {
 // residual of a 1x1 layer as {res_c channels, source pixels}: boxes {res_c, 64} (nearest-up2: the 64 source pixels under
 // 128 consecutive output pixels of one row) or {res_c, 128} (same resolution)
 static bool thin_tensor_map_r(const iea_conv_desc* d, CUtensorMap* tm) {
-  encode_tiled_fn enc = tma_encoder();
+  tc::encode_tiled_fn enc = tc::tma_encoder();
   const bool up2 = d->res_mode == IEA_IN_UP2;
   if (!enc || !d->res || d->res_dtype != IEA_BF16 || d->res_ld % 8 || ((uintptr_t)d->res & 15)) return false;
   if ((d->res_c != 16 && d->res_c != 32) || d->res_c > d->cout) return false;
@@ -721,7 +701,7 @@ static bool thin_tensor_map_r(const iea_conv_desc* d, CUtensorMap* tm) {
 }
 // {8 channels, patch width, 18 rows, 1 image} boxes of the NHWC input for 3x3; {8 channels, 128 pixels} for 1x1
 static bool thin_tensor_map(const iea_conv_desc* d, bool is3, int mt, CUtensorMap* tm) {
-  encode_tiled_fn enc = tma_encoder();
+  tc::encode_tiled_fn enc = tc::tma_encoder();
   if (!enc) return false;
   const cuuint64_t ld = (cuuint64_t)d->x_ld * 2;
   if (is3) {

@@ -2,6 +2,7 @@
 // alloc/mma/commit/ld, UMMA instruction and shared-memory descriptors) and the fused-prologue chunk loader.
 #pragma once
 #include "common.cuh"
+#include <cuda.h>
 
 namespace tc {
 using namespace iea;
@@ -92,6 +93,12 @@ __device__ __forceinline__ void tmem_alloc(uint32_t slot, uint32_t cols) {
 __device__ __forceinline__ void tmem_free(uint32_t base, uint32_t cols) {
   asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(base), "r"(cols));
 }
+// one lane of the (fully active) warp; warp-uniform code around it keeps the operands in uniform registers
+__device__ __forceinline__ bool elect_one() {
+  uint32_t pred;
+  asm volatile("{ .reg .pred P; elect.sync _|P, 0xffffffff; selp.u32 %0, 1, 0, P; }" : "=r"(pred));
+  return pred != 0;
+}
 __device__ __forceinline__ void bar_sync_epi() { asm volatile("bar.sync 1, 128;" ::: "memory"); }
 
 // one 16-byte chunk (8 channels starting at ci) of T(x) at conv-resolution pixel (n, ih, iw)
@@ -139,6 +146,22 @@ __device__ __forceinline__ uint4 load_chunk(const iea_conv_desc& d, int hs, int 
     }
   }
   return pack8(acc);
+}
+
+// cuTensorMapEncodeTiled through the runtime's driver entry point (the library does not link libcuda); null when the
+// driver does not provide it
+typedef CUresult (*encode_tiled_fn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
+                                    const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
+                                    CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
+inline encode_tiled_fn tma_encoder() {
+  static encode_tiled_fn fn = nullptr;
+  if (!fn) {
+    void* p = nullptr;
+    cudaDriverEntryPointQueryResult q;
+    if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q) == cudaSuccess && q == cudaDriverEntryPointSuccess)
+      fn = (encode_tiled_fn)p;
+  }
+  return fn;
 }
 
 inline bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15) == 0; }

@@ -44,7 +44,8 @@ def act_dtype():
 
 
 def conv_impl():
-    return {"auto": L.IMPL_AUTO, "generic": L.IMPL_GENERIC, "tcgen05": L.IMPL_TCGEN05, "stream": L.IMPL_TC_STREAM}[
+    return {"auto": L.IMPL_AUTO, "generic": L.IMPL_GENERIC, "tcgen05": L.IMPL_TCGEN05, "stream": L.IMPL_TC_STREAM,
+            "tc2": L.IMPL_TC2}[
         _env(b"IEA_CONV_IMPL", "IEA_CONV_IMPL", "auto")]
 
 

@@ -31,8 +31,9 @@ enum iea_act { IEA_ACT_NONE = 0, IEA_ACT_RELU = 1, IEA_ACT_TANH = 2 };
 /* convolution kernel choice (iea_conv_desc.impl): AUTO picks by shape; GENERIC forces the CUDA-core kernel;
  * TCGEN05 forces the tcgen05 kernels (an error where they reject the shape); TC_STREAM is TCGEN05 with the
  * streaming conv_tc kernel wherever it accepts the shape (the reference the other tcgen05 kernels are checked
- * against), else the resident-weight conv_tc2 kernel. */
-enum iea_impl { IEA_IMPL_AUTO = 0, IEA_IMPL_GENERIC = 1, IEA_IMPL_TCGEN05 = 2, IEA_IMPL_TC_STREAM = 3 };
+ * against), else the resident-weight conv_tc2 kernel; TC2 routes as AUTO except that the 1x1 layers conv_wide takes run
+ * on conv_tc2 (the reference conv_wide is checked against). */
+enum iea_impl { IEA_IMPL_AUTO = 0, IEA_IMPL_GENERIC = 1, IEA_IMPL_TCGEN05 = 2, IEA_IMPL_TC_STREAM = 3, IEA_IMPL_TC2 = 4 };
 
 /* ---- library ------------------------------------------------------------------ */
 int iea_version(void);
